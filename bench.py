@@ -4,6 +4,7 @@ including the LPG update, and meta-steps/s).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
                     [--config lpg_all_shortlife|tabular8|groove_mazes|talpg_es|double_oracle] [--scaling strong|weak]
+                    [--dump-outputs DIR]
 
 Default config = BASELINE configs[1]: LPG meta-gradient, env_mode all_shortlife, 512 agents x 64 workers x 20 steps x
 K = 5 updates.  A "step" is one full iteration of the reference's train loop (train.py:32-52): the meta-step
@@ -16,6 +17,10 @@ timed region, divided by the max-over-ranks device time.
 
 --impl reference times the CPU restatement of the reference (oracle/, torch CPU + numpy; the JAX reference itself cannot
 be installed in this image) on a bounded sample of the same workload.
+
+--dump-outputs DIR writes, after the timed steps, what the last timed step returned to its caller (LPG train state,
+agents, value critics, level buffer(s), metrics; rank 0's share) as DIR/<name>.npy, so that two builds can be compared
+output for output: the inputs are seeded, so the same arguments give the same inputs on every run.
 """
 import argparse
 import json
@@ -323,6 +328,64 @@ def timed_e2e(wl, steps, world):
     return ms, env_steps, _lib.H2D_BYTES[0] / steps, d2h
 
 
+DUMP_BUDGET = 64 << 20     # bytes of all dumped arrays together
+DUMP_SAMPLE = 1 << 20      # an output with more elements is dumped as a fixed, seeded sample of this many
+
+
+def output_arrays(wl):
+    """name -> array of what the last one_step() returned to its caller (rank 0's share of the agents)."""
+    from to_ued_b200.experiments.logging import _buffer_arrays, _train_state_arrays, to_host
+    out = {}
+
+    def put(prefix, tree):
+        for k, v in tree.items():
+            if isinstance(v, dict):
+                put(f"{prefix}.{k}", v)
+            else:
+                out[f"{prefix}.{k.replace('/', '.')}"] = v
+
+    put("train_state", _train_state_arrays(wl.train_state))
+    put("metrics", to_host(wl.metrics))
+    if wl.cfg["kind"] == "do":
+        put("train_buffer", _buffer_arrays(wl.train_buffer))
+        put("eval_buffer", _buffer_arrays(wl.eval_buffer))
+        out["train_nash"], out["eval_nash"] = wl.train_nash, wl.eval_nash
+        return out
+    if wl.buf is not None:                   # domain randomisation keeps no level buffer
+        put("level_buffer", _buffer_arrays(wl.buf))
+    ag = wl.agents
+    for name, ts in (("agents.actor", ag.actor_state), ("agents.critic", ag.critic_state), ("value_critics", wl.vcs)):
+        if ts is not None:                   # ES steps return no value critics
+            out[f"{name}.kernel"], out[f"{name}.step"] = ts.kernel, ts.step
+    out["agents.env_obs"], out["agents.env_state"] = ag.env_obs, ag.env_state.packed
+    out["agents.level.lifetime"], out["agents.level.buffer_id"] = ag.level.lifetime, ag.level.buffer_id
+    return out
+
+
+def dump_outputs(arrays, directory):
+    """Write every array as <directory>/<name>.npy: floats as float32 (float64 stays float64), integers and booleans as
+    float64 (exact to 2**53).  An array of more than DUMP_SAMPLE elements is written flat, as the elements at DUMP_SAMPLE
+    indices drawn with a fixed seed (the same indices for the same size)."""
+    import numpy as np
+    import torch
+    host = {}
+    for name, a in arrays.items():
+        if isinstance(a, torch.Tensor):
+            a = (a.float() if a.dtype in (torch.float16, torch.bfloat16) else a).detach().cpu().numpy()
+        a = np.asarray(a)
+        a = a.astype(np.float32 if a.dtype.kind == "f" and a.dtype != np.float64 else np.float64)
+        if a.size > DUMP_SAMPLE:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, DUMP_SAMPLE, replace=False))
+            a = a.reshape(-1)[idx]
+        host[name] = a
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_BUDGET:
+        raise SystemExit(f"--dump-outputs: {total} bytes of outputs exceed the {DUMP_BUDGET}-byte budget")
+    os.makedirs(directory, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 def run_ours(a):
     import torch
     import torch.distributed as dist
@@ -355,6 +418,9 @@ def run_ours(a):
     if clocks:
         clocks.stop_flag = True
         clocks.join(timeout=2)
+    # the graphed step returns views of its static buffers, which the untimed steps below overwrite
+    if a.dump_outputs and rank == 0:
+        dump_outputs(output_arrays(wl), a.dump_outputs)
 
     # ---- per-kernel CUDA-event times for the roofline / shares: eager enqueue (no graph), the mini-batches one after the
     #      other on one stream and no side streams, so that every launch is timed without a concurrent neighbour ----
@@ -566,7 +632,12 @@ def main():
     ap.add_argument("--no-fp32", dest="no_fp32", action="store_true", help="skip the exact-fp32 path measurement")
     ap.add_argument("--no-other-scaling", dest="no_other_scaling", action="store_true",
                     help="N > 1: skip the second (weak / strong) measurement")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR",
+                    help="after the timed steps, write the last timed step's outputs as DIR/<name>.npy (--impl ours; "
+                         "bench_outputs/ is git-ignored for this)")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if a.impl == "reference":
         run_reference(a)
     else:
