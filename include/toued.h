@@ -315,9 +315,18 @@ int toued_gru_forward_tc_multi(const float* x, const uint8_t* done, const float*
 /* Pack Wh into the bf16 SW128 chunk images of the tensor-core reverse pass (384 KiB).               */
 int toued_pack_wh_backward(const float* lpg_params, void* whb_img, void* stream);
 /* Scaled fp16 reverse pass.  The reverse pass is linear in the cotangents (d_pi_hat, d_y_hat), which are far below
- * fp16's range: toued_cotangent_max writes max |cotangent| of a launch (bit pattern of a float) to cotangent_max u32[1],
- * the tensor-core reverse kernels derive a power of two S from it, run on S x cotangents with fp16 operands (saturating
- * conversions) and fp32 accumulation, and the consumers divide S back out.  cotangent_max == NULL means S = 1.    */
+ * fp16's range: the tensor-core reverse kernels derive a power of two S from max |cotangent|, run on S x cotangents
+ * with fp16 operands (saturating conversions) and fp32 accumulation, and the consumers divide S back out.
+ * cotangent_max u32[2] of one launch = {max, status}:
+ *   [0] max |cotangent| as the bit pattern of a float, +inf if any cotangent is inf or NaN (then S = 1);
+ *       written by toued_cotangent_max, which resets this word only;
+ *   [1] status bits, OR-ed in and never cleared by a kernel (the caller zeroes the word): a set bit means the result of
+ *       the launch may be wrong.  TOUED_STATUS_NONFINITE_COT: toued_cotangent_max saw an inf / NaN cotangent.
+ *       TOUED_STATUS_FP16_RANGE: toued_gru_backward_tc or toued_lpg_wgrad_tc met an fp16 operand with |S v| > 65504
+ *       (saturated: the carry grew past ~2^12 x max |cotangent| along the chain) or non-finite.
+ * cotangent_max == NULL means S = 1 and no status.                                                            */
+#define TOUED_STATUS_NONFINITE_COT 1u
+#define TOUED_STATUS_FP16_RANGE 2u
 int toued_cotangent_max(const float* d_pi_hat, const float* d_y_hat, int n_agents, int n_workers, int rollout_len,
                         uint32_t* cotangent_max, void* stream);
 /* Tensor-core BPTT (reverse of toued_gru_forward_tc).  Reads h16 / fac saved by the forward; writes, in units of S,
@@ -325,7 +334,7 @@ int toued_cotangent_max(const float* d_pi_hat, const float* d_y_hat, int n_agent
  *   dl f32[L][R][8] head-logit cotangents, dx f32[L][R][2] (d pyt, d pyt1)                          */
 int toued_gru_backward_tc(const uint8_t* done, const float* lpg_params, const void* whb_img,
                           const void* h16, const void* fac, const float* y_hat, const float* d_pi_hat,
-                          const float* d_y_hat, void* dgimg, float* dl, float* dx, const uint32_t* cotangent_max,
+                          const float* d_y_hat, void* dgimg, float* dl, float* dx, uint32_t* cotangent_max,
                           int n_agents, int n_workers, int rollout_len, int lifetime_conditioning, void* stream);
 /* Tensor-core weight gradients from the token tile images (hpimg from the forward, dgimg from the
  * backward) + streaming small gradients; partial areas of the toued_lpg_wgrad workspace.             */
@@ -333,7 +342,7 @@ int toued_wgrad_tc_splits(void);
 int toued_wgrad_tc_small_splits(void);
 int toued_lpg_wgrad_tc(const void* hpimg, const void* dgimg, const void* ximg, const void* h16,
                        const float* d_pi_hat, const float* dl, float* wh_partials, float* small_partials,
-                       const uint32_t* cotangent_max, int n_agents, int n_workers, int rollout_len, int accumulate,
+                       uint32_t* cotangent_max, int n_agents, int n_workers, int rollout_len, int accumulate,
                        void* stream);
 
 #ifdef __cplusplus

@@ -69,9 +69,10 @@ def init_lpg_params(layout: LPGLayout, seed: int = 0) -> np.ndarray:
     return np.concatenate([p[name].reshape(-1) for name, _ in layout.shapes]).astype(np.float32)
 
 
-def lpg_forward(layout: LPGLayout, flat, r, d, pi, yt, yt1, step, lifetime):
+def lpg_forward(layout: LPGLayout, flat, r, d, pi, yt, yt1, step, lifetime, hidden=None):
     """models/lpg.py:48-85.  r, d, pi: [B, L]; yt, yt1: [B, L, Y]; step, lifetime: [B] (per
-    sequence).  Returns pi_hat [B, L], y_hat [B, L, Y]."""
+    sequence).  Returns pi_hat [B, L], y_hat [B, L, Y].  ``hidden`` (a list, optional) receives the
+    hidden states h_t [B, H] in time order, e.g. to read their gradients."""
     P = layout.unpack(flat)
     H = layout.H
     dt = flat.dtype
@@ -98,6 +99,8 @@ def lpg_forward(layout: LPGLayout, flat, r, d, pi, yt, yt1, step, lifetime):
         ng = torch.tanh(gi[:, t, 2 * H:] + rg * (gh[:, 2 * H:] + P["bhn"]))
         h = (1.0 - zg) * ng + zg * h
         outs[t] = h
+    if hidden is not None:
+        hidden.extend(outs)
     y = torch.relu(torch.stack(outs, dim=1))                # [B, L, H]
     pi_hat = y @ P["w_pi"] + P["b_pi"]                      # Dense(1), squeezed
     y_hat = torch.softmax(y @ P["W_y"] + P["b_y"], dim=-1)

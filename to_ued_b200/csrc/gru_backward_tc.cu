@@ -12,8 +12,10 @@
 // bits without ever leaving tensor memory.
 // Scaled arithmetic (tc.cuh, "scaled fp16 operands"): the kernel multiplies the incoming cotangents by the power of two
 // S derived from `cotmax` and everything downstream -- carry, dG, dl, dx -- is in units of S; the consumers
-// (toued_lpg_wgrad_tc, toued_lpg_wgrad_embed) take S back out.  Round 1 used bf16 operands (8 significant bits; the
-// rounding of Wh is systematic over all tokens) and left 0.6-1.6e-2 of error on the GRU weight blocks of the meta-gradient.
+// (toued_lpg_wgrad_tc, toued_lpg_wgrad_embed) take S back out.  A dG or z*dh value that leaves fp16's range (the
+// conversion saturates it) or is not finite sets TOUED_STATUS_FP16_RANGE in cotmax[1]: the result is then unreliable.
+// Round 1 used bf16 operands (8 significant bits; the rounding of Wh is systematic over all tokens) and left 0.6-1.6e-2
+// of error on the GRU weight blocks of the meta-gradient.
 // Outputs for the weight-gradient kernels: S * dG (dar, daz, dhn, dan) as an fp16 token-tile image,
 // the head-logit cotangents S * dl and S * (d pyt, d pyt1).
 #include "tc.cuh"
@@ -77,7 +79,7 @@ gru_backward_tc_kernel(const uint8_t* __restrict__ done, const float* __restrict
                        const __half* __restrict__ fac, const float* __restrict__ y_hat,
                        const float* __restrict__ d_pi_hat, const float* __restrict__ d_y_hat,
                        unsigned char* __restrict__ dgimg, float* __restrict__ dl_out, float* __restrict__ dx,
-                       const uint32_t* __restrict__ cotmax, int R, int L, int W) {
+                       uint32_t* __restrict__ cotmax, int R, int L, int W) {
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     // (offset arithmetic on the __shared__ array, not an integer round trip: the compiler keeps the shared
     //  address space and emits LDS / STS instead of generic LD / ST)
@@ -258,6 +260,12 @@ gru_backward_tc_kernel(const uint8_t* __restrict__ done, const float* __restrict
         const int rsafe = rv ? row : 0;
         const int n_ag = rsafe / W, w_ag = rsafe % W;
         uint32_t ait = 0;
+        // Some fp16 operand of this thread left fp16's range (the conversion saturated it) or was not finite: reported in
+        // cotmax[1].  Two checks per element cover all five operands: |cz| <= |dh|, |gan|, |ghn| <= |dh| and
+        // |gz| <= |dh| / 2 (z, r, n, h' in their ranges), so |dh| bounds all but gr; a NaN anywhere in the chain (dh, or
+        // a saved gate) reaches gr through gan and ghn.  A NaN stays in the running maximum.  Checking dh rather than
+        // z * dh also reports a carry grown past 65504 / S where z happens to be small.
+        float range_max = 0.0f;                  // NaN-propagating running max of |dh|, |gr|
         const uint32_t sS_u32 = smem_u32(sS), sC_u32 = smem_u32(sC);
         const float S = cotmax ? cot_scale_from_max(*cotmax) : 1.0f;      // power of two: scaling is exact
         // ---- software pipeline: the factor loads of the next 8-unit chunk and the head cotangents of the
@@ -385,6 +393,7 @@ gru_backward_tc_kernel(const uint8_t* __restrict__ done, const float* __restrict
                         gr[e] = ghn[e] * hn_[e] * (1.0f - gr_[e]);
                         gz[e] = dh * (nd_hp * hx[e] - gn_[e]) * zz[e] * omz;
                         cz[e] = dh * zz[e];
+                        range_max = fmax3_nan(range_max, fabsf(dh), fabsf(gr[e]));
                         {
                             const float4 w0 = *reinterpret_cast<const float4*>(sWi + u * 4);
                             const float2 w1 = *reinterpret_cast<const float2*>(sWi2 + u * 2);
@@ -441,6 +450,7 @@ gru_backward_tc_kernel(const uint8_t* __restrict__ done, const float* __restrict
             }
             asm volatile("bar.sync 1, %0;" ::"n"(BT_EW * 32) : "memory");
         }
+        if (__any_sync(0xffffffffu, !(range_max <= 65504.0f)) && lane == 0 && cotmax) atomicOr(cotmax + 1, TOUED_STATUS_FP16_RANGE);
     }
     tc_fence_before();
     __syncthreads();
@@ -453,7 +463,7 @@ static size_t gru_bwd_tc_smem() {
 
 extern "C" int toued_gru_backward_tc(const uint8_t* done, const float* lpg_params, const void* whb_img,
                                      const void* h16, const void* fac, const float* y_hat, const float* d_pi_hat,
-                                     const float* d_y_hat, void* dgimg, float* dl, float* dx, const uint32_t* cotangent_max,
+                                     const float* d_y_hat, void* dgimg, float* dl, float* dx, uint32_t* cotangent_max,
                                      int n_agents, int n_workers, int rollout_len, int lifetime_conditioning, void* stream) {
     const int R = n_agents * n_workers;
     TOUED_CHECK(R > 0 && rollout_len > 0, "toued_gru_backward_tc: empty problem");

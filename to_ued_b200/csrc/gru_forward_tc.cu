@@ -369,9 +369,10 @@ gru_forward_tc_kernel(const float* __restrict__ x, const uint8_t* __restrict__ d
                     const int u = u0 + e;
                     // The epilogue is bound by the MUFU pipe (16 results / clk / SM; 6 MUFU operations per unit with three
                     // ex2 + rcp activations).  The two sigmoids share ONE reciprocal: inv = 1/(a b), r = b inv, z = a inv
-                    // (exponents clamped at 60 so that the product stays finite; sigmoid is 0 to fp32 there anyway).
-                    const float ea = ex2_approx(fminf(-1.4426950408889634f * ar[e], 60.0f));
-                    const float eb = ex2_approx(fminf(-1.4426950408889634f * az[e], 60.0f));
+                    // (exponents clamped at 60 so that the product stays finite; sigmoid is 0 to fp32 there anyway; the clamp
+                    // keeps a NaN pre-activation NaN).
+                    const float ea = ex2_approx(fmin_nan(-1.4426950408889634f * ar[e], 60.0f));
+                    const float eb = ex2_approx(fmin_nan(-1.4426950408889634f * az[e], 60.0f));
                     const float da = 1.0f + ea, db = 1.0f + eb;
                     const float inv = rcp_approx(da * db);
                     rr[e] = inv * db;                                     // input projection + bias already inside
@@ -397,7 +398,7 @@ gru_forward_tc_kernel(const float* __restrict__ x, const uint8_t* __restrict__ d
                     uint4 rl4;
                     const __half2 z2 = __float2half2_rn(0.0f);
                     const __half2* hs = reinterpret_cast<const __half2*>(&hpk);
-                    __half2 r0 = __hmax2(hs[0], z2), r1 = __hmax2(hs[1], z2), r2 = __hmax2(hs[2], z2), r3 = __hmax2(hs[3], z2);
+                    __half2 r0 = __hmax2_nan(hs[0], z2), r1 = __hmax2_nan(hs[1], z2), r2 = __hmax2_nan(hs[2], z2), r3 = __hmax2_nan(hs[3], z2);
                     rl4.x = *reinterpret_cast<uint32_t*>(&r0); rl4.y = *reinterpret_cast<uint32_t*>(&r1);
                     rl4.z = *reinterpret_cast<uint32_t*>(&r2); rl4.w = *reinterpret_cast<uint32_t*>(&r3);
                     tmem_st4(tmem_base + ((uint32_t)(q * 32) << 16) + FT_TTILE + sb * 8 + hf * 4, rl4);

@@ -667,20 +667,26 @@ extern "C" int toued_sgd_clip(float* params, const float* grad, float* sqnorm_sc
 // ------------------------------------------------------------------------------------------------
 // max |cotangent| of one reverse-pass launch (d pi_hat f32[n_tok], d y_hat f32[n_tok][8]) as the bit pattern of a
 // non-negative float (integer order == float order, so atomicMax is exact and order-independent): the tensor-core
-// reverse kernels derive their power-of-two operand scale from it (tc.cuh::cot_scale_from_max).
+// reverse kernels derive their power-of-two operand scale from it (tc.cuh::cot_scale_from_max).  The maximum is taken
+// over the bit patterns of |v|, in which NaN sorts above +inf: any non-finite cotangent gives +inf (S = 1) and sets
+// TOUED_STATUS_NONFINITE_COT in out_bits[1] (fmaxf would skip a NaN and report the finite maximum).
 __global__ void cot_max_kernel(const float* __restrict__ d_pi_hat, const float* __restrict__ d_y_hat, size_t n_tok,
                                uint32_t* __restrict__ out_bits) {
-    float m = 0.f;
+    uint32_t m = 0u;
     const size_t stride = (size_t)gridDim.x * blockDim.x;
-    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_tok; i += stride) m = fmaxf(m, fabsf(d_pi_hat[i]));
-    const float4* y4 = reinterpret_cast<const float4*>(d_y_hat);
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_tok; i += stride)
+        m = max(m, __float_as_uint(d_pi_hat[i]) & 0x7FFFFFFFu);
+    const uint4* y4 = reinterpret_cast<const uint4*>(d_y_hat);
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < 2 * n_tok; i += stride) {
-        const float4 v = y4[i];
-        m = fmaxf(m, fmaxf(fmaxf(fabsf(v.x), fabsf(v.y)), fmaxf(fabsf(v.z), fabsf(v.w))));
+        const uint4 v = y4[i];
+        m = max(m, max(max(v.x & 0x7FFFFFFFu, v.y & 0x7FFFFFFFu), max(v.z & 0x7FFFFFFFu, v.w & 0x7FFFFFFFu)));
     }
 #pragma unroll
-    for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
-    if ((threadIdx.x & 31) == 0 && m > 0.f) atomicMax(out_bits, __float_as_uint(m));
+    for (int o = 16; o > 0; o >>= 1) m = max(m, __shfl_xor_sync(0xffffffffu, m, o));
+    if ((threadIdx.x & 31) == 0 && m > 0u) {
+        atomicMax(out_bits, min(m, 0x7F800000u));
+        if (m >= 0x7F800000u) atomicOr(out_bits + 1, TOUED_STATUS_NONFINITE_COT);
+    }
 }
 
 extern "C" int toued_cotangent_max(const float* d_pi_hat, const float* d_y_hat, int n_agents, int n_workers, int rollout_len,
@@ -688,7 +694,7 @@ extern "C" int toued_cotangent_max(const float* d_pi_hat, const float* d_y_hat, 
     const size_t n_tok = (size_t)n_agents * n_workers * rollout_len;
     TOUED_CHECK(n_tok > 0 && out_bits != nullptr, "toued_cotangent_max: bad arguments");
     cudaStream_t st = (cudaStream_t)stream;
-    TOUED_CUDA(cudaMemsetAsync(out_bits, 0, sizeof(uint32_t), st));
+    TOUED_CUDA(cudaMemsetAsync(out_bits, 0, sizeof(uint32_t), st));     // word 0 only: the status word is sticky
     cot_max_kernel<<<296, 256, 0, st>>>(d_pi_hat, d_y_hat, n_tok, out_bits);
     TOUED_LAUNCH_CHECK();
     return 0;

@@ -53,6 +53,14 @@ __device__ __forceinline__ float sigmoid_mufu(float x) { return fmaf(0.5f, tanh_
 __device__ __forceinline__ float sigmoid_fast(float x) { return rcp_approx(1.0f + ex2_approx(-1.4426950408889634f * x)); }
 __device__ __forceinline__ float tanh_fast(float x) { return fmaf(2.0f, rcp_approx(1.0f + ex2_approx(-2.8853900817779268f * x)), -1.0f); }
 
+// min / max that return NaN when an operand is NaN (fminf / fmaxf return the other operand): one FMNMX, like fminf,
+// and the same result on non-NaN operands.  A NaN pre-activation then reaches pi_hat / y_hat instead of turning finite.
+__device__ __forceinline__ float fmin_nan(float a, float b) { float r; asm("min.NaN.f32 %0, %1, %2;" : "=f"(r) : "f"(a), "f"(b)); return r; }
+__device__ __forceinline__ float fmax_nan(float a, float b) { float r; asm("max.NaN.f32 %0, %1, %2;" : "=f"(r) : "f"(a), "f"(b)); return r; }
+__device__ __forceinline__ float fmax3_nan(float a, float b, float c) {
+    float r; asm("max.NaN.f32 %0, %1, %2, %3;" : "=f"(r) : "f"(a), "f"(b), "f"(c)); return r;
+}
+
 // softmax over C values (true expf; float path, tolerance-checked)
 template <int C>
 __device__ __forceinline__ void softmax_c(const float (&z)[C], float (&p)[C]) {

@@ -143,8 +143,8 @@ __device__ __forceinline__ void embed_mlp2(const float (&y0)[LPG_Y], const float
             a1 = fmaf(y1[i], wgt, a1);
         }
         const float w1 = sp[LPG_Y * LPG_E + LPG_E + e];
-        out0 = fmaf(fmaxf(a0, 0.0f), w1, out0);
-        out1 = fmaf(fmaxf(a1, 0.0f), w1, out1);
+        out0 = fmaf(fmax_nan(a0, 0.0f), w1, out0);             // relu that keeps NaN (fmaxf would drop it)
+        out1 = fmaf(fmax_nan(a1, 0.0f), w1, out1);
     }
 }
 
@@ -389,7 +389,7 @@ gru_forward_kernel(const float* __restrict__ x, const uint8_t* __restrict__ done
 #pragma unroll
             for (int c = 0; c < 1 + LPG_Y; ++c) hacc[c] = 0.0f;
             for (int k = part * 64; k < part * 64 + 64; ++k) {
-                const float yv = fmaxf(hB[rl * GF_HS + k], 0.0f);
+                const float yv = fmax_nan(hB[rl * GF_HS + k], 0.0f);     // relu that keeps NaN
                 hacc[0] = fmaf(yv, swp[k], hacc[0]);
 #pragma unroll
                 for (int c = 0; c < LPG_Y; ++c) hacc[1 + c] = fmaf(yv, sWy[k * LPG_Y + c], hacc[1 + c]);

@@ -206,6 +206,7 @@ __device__ __forceinline__ void mbar_wait_cluster(uint64_t* bar, uint32_t parity
 // operands everywhere (dG, z * dh, Wh, h', x: 8x finer than bf16; h' is even exact, it IS fp16), convert with saturation,
 // and multiply their fp32 results by 1 / S when they leave the kernel.  S puts the largest cotangent at [2^3, 2^4): a
 // factor 2^12 of headroom for growth along the 20-step chain before saturation, ~2^-27 of the maximum before underflow.
+// A saturated or non-finite operand is not corrected but reported in the launch's status word (include/toued.h).
 __device__ __forceinline__ float cot_scale_from_max(uint32_t max_bits) {
     if (max_bits == 0u || max_bits >= 0x7F800000u) return 1.0f;           // no signal, or inf / nan: leave unscaled
     const int e = (int)(max_bits >> 23) - 127;                            // floor(log2(max))

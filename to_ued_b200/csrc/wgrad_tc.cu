@@ -252,7 +252,7 @@ wgrad_heads_stream_kernel(const __half* __restrict__ h16, const float* __restric
 #pragma unroll
         for (int e2 = 0; e2 < 4; ++e2) {
             const float2 f = __half22float2(hh[e2]);
-            const float y0 = fmaxf(f.x, 0.0f), y1 = fmaxf(f.y, 0.0f);
+            const float y0 = fmax_nan(f.x, 0.0f), y1 = fmax_nan(f.y, 0.0f);       // relu that keeps NaN
 #pragma unroll
             for (int i = 0; i < 9; ++i) { acc[2 * e2][i] = fmaf(y0, dv[i], acc[2 * e2][i]); acc[2 * e2 + 1][i] = fmaf(y1, dv[i], acc[2 * e2 + 1][i]); }
         }
@@ -300,7 +300,7 @@ constexpr int HM_STAGE = HM_A + HM_RAW + HM_B;            // 19584 B (multiple o
 constexpr int HM_THREADS = 192;
 __global__ void __launch_bounds__(HM_THREADS, 1)
 wgrad_heads_mma_kernel(const __half* __restrict__ h16, const float* __restrict__ d_pi_hat, const float* __restrict__ dl,
-                       float* __restrict__ partial, const uint32_t* __restrict__ cotmax, int R, int L, int blocks_per_split,
+                       float* __restrict__ partial, uint32_t* __restrict__ cotmax, int R, int L, int blocks_per_split,
                        int accumulate) {
     extern __shared__ __align__(1024) unsigned char hm_raw[];
     unsigned char* smem = hm_raw + ((128u - (smem_u32(hm_raw) & 127u)) & 127u);
@@ -369,6 +369,7 @@ wgrad_heads_mma_kernel(const __half* __restrict__ h16, const float* __restrict__
 #pragma unroll
         for (int i = 0; i < 9; ++i) hb[i] = 0.f;
         const float S = cotmax ? cot_scale_from_max(*cotmax) : 1.0f, inv_s = 1.0f / S;
+        bool range_bad = false;                   // an operand was clamped to fp16's range or is not finite (cotmax[1])
         for (int i = 0; i < nblk; ++i) {
             const int s = i % HM_NS;
             mbar_wait(&full[s], (i / HM_NS) & 1);
@@ -381,7 +382,7 @@ wgrad_heads_mma_kernel(const __half* __restrict__ h16, const float* __restrict__
                 uint4 raw = *pp;
                 __half2* hh = reinterpret_cast<__half2*>(&raw);
 #pragma unroll
-                for (int e = 0; e < 4; ++e) hh[e] = __hmax2(hh[e], z2);
+                for (int e = 0; e < 4; ++e) hh[e] = __hmax2_nan(hh[e], z2);
                 *pp = raw;
             }
             if (warp == 0) {
@@ -393,7 +394,9 @@ wgrad_heads_mma_kernel(const __half* __restrict__ h16, const float* __restrict__
                 float hi[9], lo[9];
 #pragma unroll
                 for (int j = 0; j < 9; ++j) {
-                    hi[j] = __half2float(__float2half_rn(fminf(fmaxf(dv[j], -65504.0f), 65504.0f)));
+                    // (a NaN passes the clamp instead of becoming -65504)
+                    range_bad |= !(fabsf(dv[j]) <= 65504.0f);
+                    hi[j] = __half2float(__float2half_rn(fmin_nan(fmax_nan(dv[j], -65504.0f), 65504.0f)));
                     lo[j] = dv[j] - hi[j];
                     hb[j] += dv[j];
                 }
@@ -408,6 +411,7 @@ wgrad_heads_mma_kernel(const __half* __restrict__ h16, const float* __restrict__
             __syncwarp();
             if (lane == 0) mbar_arrive(&ready[s]);
         }
+        if (warp == 0 && __any_sync(0xffffffffu, range_bad) && lane == 0 && cotmax) atomicOr(cotmax + 1, TOUED_STATUS_FP16_RANGE);
         // ---- epilogue: TMEM lane = unit within the 128-unit half ----
         mbar_wait(&done_bar, 0);
         tc_fence_after();
@@ -839,7 +843,7 @@ extern "C" int toued_wgrad_tc_small_splits(void) { return HT_SPLITS; }
 
 extern "C" int toued_lpg_wgrad_tc(const void* hpimg, const void* dgimg, const void* ximg, const void* h16,
                                   const float* d_pi_hat, const float* dl, float* wh_partials, float* small_partials,
-                                  const uint32_t* cotangent_max, int n_agents, int n_workers, int rollout_len, int accumulate,
+                                  uint32_t* cotangent_max, int n_agents, int n_workers, int rollout_len, int accumulate,
                                   void* stream) {
     const int R = n_agents * n_workers, L = rollout_len;
     TOUED_CHECK(R > 0 && L > 0, "toued_lpg_wgrad_tc: empty problem");

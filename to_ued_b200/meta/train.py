@@ -69,8 +69,9 @@ class MetaGradWorkspace:
         if self.tape.precision == "tc":
             Rp = (R + 63) // 64 * 64
             self.whb_img = torch.empty(256 * 768, dtype=torch.float16, device=device)
-            # max |cotangent| of every update's reverse launch (scaled fp16 operands, csrc/tc.cuh)
-            self.cotmax = torch.zeros(K, dtype=torch.int32, device=device)
+            # {max |cotangent|, status bits} of every update's reverse launch (scaled fp16 operands, csrc/tc.cuh;
+            # include/toued.h toued_cotangent_max): the status words are sticky, read by reverse_status()
+            self.cotmax = torch.zeros((K, 2), dtype=torch.int32, device=device)
             # fp16 token-tile image of S * (dar, daz, dhn, dan): 16 column groups of 64
             # (double-buffered over the update index like the cotangents: the weight-gradient GEMMs of update k run on
             #  their own stream next to the BPTT of update k-1)
@@ -93,6 +94,22 @@ def _workspace(n, w, L, D, K, P, device, slot=0) -> MetaGradWorkspace:
     if ws is None:
         ws = _WS_CACHE[key + (slot,)] = MetaGradWorkspace(n, w, L, D, K, P, device)
     return ws
+
+
+def reverse_status(reset=False):
+    """OR of the status words of the tensor-core reverse passes run since the workspaces were created (or last reset):
+    an int32 device tensor, 0 when every meta-gradient came out clean.  Bit TOUED_STATUS_NONFINITE_COT (1): a cotangent
+    was inf / NaN; bit TOUED_STATUS_FP16_RANGE (2): an fp16 operand of the reverse pass saturated or was not finite, so
+    the meta-gradient may be wrong (include/toued.h).  Only the tensor-core path (GRU_PRECISION "tc") sets bits.  No
+    host synchronisation unless the caller reads the value."""
+    st = torch.zeros((), dtype=torch.int32, device="cuda")
+    for ws in _WS_CACHE.values():
+        if getattr(ws, "cotmax", None) is not None:
+            for w in ws.cotmax[:, 1]:
+                st = st | w
+            if reset:
+                ws.cotmax[:, 1].zero_()
+    return st
 
 
 def _eval_stream(device):
@@ -320,7 +337,7 @@ def lpg_meta_grad_train_step(rng, lpg_train_state: LPGTrainState, agent_states: 
             if k + 2 <= K - 1:
                 st.wait_event(ev["wg"][k + 2])              # the cotangent buffer is free again
             _agent_backward(ws, tape, k, buf, _lib.stream_ptr())
-            _lib.call("toued_cotangent_max", p(ws.d_pi_hat2[buf]), p(ws.d_y_hat2[buf]), nb, W, L, p(ws.cotmax[k:k + 1]),
+            _lib.call("toued_cotangent_max", p(ws.d_pi_hat2[buf]), p(ws.d_y_hat2[buf]), nb, W, L, p(ws.cotmax[k]),
                       _lib.stream_ptr())
             ev["ab"][k].record(st)
         with torch.cuda.stream(streams[slot]):
@@ -332,7 +349,7 @@ def lpg_meta_grad_train_step(rng, lpg_train_state: LPGTrainState, agent_states: 
                 st.wait_event(ev["wg"][k + 2])              # ... and so have the dG image and dl [k & 1]
             _lib.call("toued_gru_backward_tc", p(tape.done[k]), p(lpg), p(ws.whb_img), p(tape.h16[k]),
                       p(tape.fac[k]), p(tape.y_hat[k]), p(ws.d_pi_hat2[buf]), p(ws.d_y_hat2[buf]), p(ws.dgimg2[buf]), p(ws.dl2[buf]),
-                      p(ws.dx2[buf]), p(ws.cotmax[k:k + 1]), nb, W, L, cond, s)
+                      p(ws.dx2[buf]), p(ws.cotmax[k]), nb, W, L, cond, s)
             ev["bwd"][k].record(st)
             _phase(f"bwd{k}", mb, st)
         with torch.cuda.stream(wg_streams[slot]):
@@ -340,14 +357,14 @@ def lpg_meta_grad_train_step(rng, lpg_train_state: LPGTrainState, agent_states: 
             st.wait_event(ev["bwd"][k])
             _lib.call("toued_lpg_wgrad_tc", p(tape.hpimg[k]), p(ws.dgimg2[buf]), p(tape.ximg[k]), p(tape.h16[k]),
                       p(ws.d_pi_hat2[buf]), p(ws.dl2[buf]), p(ws.partials), p(ws.partials[ws.off_small:]),
-                      p(ws.cotmax[k:k + 1]), nb, W, L, 0 if first else 1, _lib.stream_ptr())
+                      p(ws.cotmax[k]), nb, W, L, 0 if first else 1, _lib.stream_ptr())
             ev["wg"][k].record(st)
             _phase(f"wgrad{k}", mb, st)
         with torch.cuda.stream(em_streams[slot]):
             st = em_streams[slot]
             st.wait_event(ev["bwd"][k])
             _lib.call("toued_lpg_wgrad_embed", p(tape.obs[k]), p(tape.done[k]), p(tape.critic[k]), p(lpg),
-                      p(ws.dx2[buf]), p(ws.partials), p(ws.cotmax[k:k + 1]), nb, W, L, D, cond, 0 if first else 1,
+                      p(ws.dx2[buf]), p(ws.partials), p(ws.cotmax[k]), nb, W, L, D, cond, 0 if first else 1,
                       _lib.stream_ptr())
             ev["em"][k].record(st)
 

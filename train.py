@@ -94,6 +94,12 @@ def run_training_experiment(args):
     train_fn = make_train(args, rank, world)
     metrics, train_state, level_buffer = train_fn(prng.PRNGKey(args.seed))
     torch.cuda.synchronize()
+    from to_ued_b200.meta.train import reverse_status
+    status = int(reverse_status())
+    if status:
+        print(f"[to_ued_b200] warning (rank {rank}): the tensor-core reverse pass reported status {status:#x} "
+              "(1: inf / NaN cotangent, 2: fp16 operand saturated or not finite); some meta-gradients may be wrong. "
+              "TOUED_GRU_PRECISION=fp32 runs the exact-fp32 reverse pass.", file=sys.stderr)
     if rank == 0:
         print([_to_float(m) for m in metrics])
         if args.log:                                 # train.py:68-69
