@@ -240,6 +240,14 @@ int toued_generate_levels_desc_bytes(void);
 int toued_generate_levels(const void* gen_desc, const uint32_t* keys, const int32_t* buffer_ids, void* levels_out,
                           int32_t* lifetimes_out, int n_levels, void* stream);
 
+/* ---- optimal return (environments/gridworld/gridworld.py:253-323 optimal_return) ------------------- */
+/* out f64[n_levels] = the optimal expected undiscounted first-episode return of each LevelRec over `horizon` steps
+ * (the level's max_steps caps the episode): exact finite-horizon DP over (cell, exists mask) in fp64 with a fixed
+ * operation order, bitwise reproducible and independent of the batch.  max_n_objs <= 5, max_grid_size^2 <= 255;
+ * a record outside those bounds gives NaN.                                                                  */
+int toued_optimal_return(const void* levels, int n_levels, int horizon, int max_grid_size, int max_n_objs,
+                         double* out, void* stream);
+
 /* ---- double-oracle Nash solver (environments/nash_sampler.py:24-58, util/projection.py:9-38) ------ */
 /* game f32[n][n] (row player x minimises x^T G y), supports = first x_nz / y_nz coordinates, n <= 1024.
  * Averaged iterates of num_iters projected-gradient steps (reference: 10,000 steps, lr 0.01).        */
@@ -293,7 +301,7 @@ int toued_tc_gemm_mn2_test(const float* A, const float* B, void* scratch_img, fl
  * forward streams (wh_img: 16 x 26 KiB = 416 KiB, once per meta-step).                              */
 int toued_pack_wh_forward(const float* lpg_params, void* wh_img, int lifetime_conditioning, void* stream);
 /* Tensor-core version of toued_gru_forward (models/lpg.py:11-30,77-84): fp16 operands, fp32
- * accumulation in TMEM.  Saved for the reverse pass (NULL to skip):
+ * accumulation in TMEM.  Saved for the reverse pass (NULL to skip; h16 may be NULL only when fac and hpimg are):
  *   h16   f16, RB32 layout [L][ceil(R/32)][32 chunks][32 rows][8 units] (csrc/tc.cuh::rb32_index)   h_t
  *   fac   f16 [L][R/32][4 planes][32 chunks][32 rows][8]: the gates r, z, n and hn = Whn h' + bhn as RB32 blocks with
  *         the planes interleaved per (t, 32-row block); the sign bits of the z plane carry relu'(h_t) (set: h_t <= 0).

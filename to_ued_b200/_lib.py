@@ -90,6 +90,7 @@ SIGNATURES = {
     "toued_key_split": [_P, _I, _I, _I, _I, _P, _P],
     "toued_key_chain": [_P, _I, _I, _P, _P, _P],
     "toued_gru_forward_tc": [_P] * 9 + [_I] * 4 + [_P],
+    "toued_optimal_return": [_P] + [_I] * 4 + [_P, _P],
 }
 
 

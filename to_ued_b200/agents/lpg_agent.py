@@ -67,7 +67,8 @@ class Tape:
             f16 = torch.float16
             Rp = (R + 63) // 64 * 64
             R32 = (R + 31) // 32 * 32                         # RB32 layout pads rows to blocks of 32
-            self.h16 = None if per_agent_params else torch.empty((ka, L, R32, 256), dtype=f16, device=dev)
+            # h16 (h_t for the reverse pass) only on recording tapes: inference never reads it
+            self.h16 = torch.empty((ka, L, R32, 256), dtype=f16, device=dev) if self.record and not per_agent_params else None
             self.fac = torch.empty((ka, 4, L, R32, 256), dtype=f16, device=dev) if self.record else None
             # bf16 token-tile images (rows >= R of a partial 64-token block stay zero)
             self.hpimg = torch.zeros((ka, L * Rp * 256 * 2), dtype=torch.uint8, device=dev) if self.record else None
@@ -163,7 +164,7 @@ def lpg_agent_train_step(k, tape: Tape, levels, step, lpg_params, lifetime_condi
                   N, W, L, int(lifetime_conditioning), int(lpg_stride), s)
     else:
         _lib.call("toued_gru_forward_tc", p(tape.x[a]), p(tape.done[r]), p(lpg_params), p(tape.wh_img),
-                  p(tape.h16[a]), p(tape.fac[a]) if tape.fac is not None else None,
+                  p(tape.h16[a]) if tape.h16 is not None else None, p(tape.fac[a]) if tape.fac is not None else None,
                   p(tape.hpimg[a]) if tape.hpimg is not None else None, p(tape.pi_hat[a]), p(tape.y_hat[a]),
                   N, W, L, int(lifetime_conditioning), s)
     _mark("gru_fwd")

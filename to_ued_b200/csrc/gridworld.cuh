@@ -31,6 +31,21 @@ __device__ __forceinline__ StepRand<O> env_step_rand(Key k_env) {
     return r;
 }
 
+// _get_next_pos (gridworld.py:138-146) on its own: the same clamping and wall test as the first block of
+// env_step_apply, for callers that enumerate moves instead of simulating them (csrc/optimal_return.cu).
+__device__ __forceinline__ int env_next_pos(const LevelRec& lev, int pos, int a) {
+    const int gsz = lev.grid_size;
+    const int col = pos % gsz;
+    int step = 0;
+    if (a == 0 && pos >= gsz) step = -gsz;
+    else if (a == 1 && pos < gsz * (gsz - 1)) step = gsz;
+    else if (a == 2 && col != 0) step = -1;
+    else if (a == 3 && col != gsz - 1) step = 1;
+    const int nxt = pos + step;
+    const bool blocked = (lev.walls[nxt >> 5] >> (nxt & 31)) & 1u;
+    return blocked ? pos : nxt;
+}
+
 // One auto-resetting transition.  Returns reward; sets done.
 template <int O>
 __device__ __forceinline__ float env_step_apply(const LevelRec& lev, const StepRand<O>& rnd, int a,

@@ -508,7 +508,8 @@ extern "C" int toued_gru_forward_tc(const float* x, const uint8_t* done, const f
                                     void* h16, void* fac, void* hpimg, float* pi_hat, float* y_hat, int n_agents,
                                     int n_workers, int rollout_len, int lifetime_conditioning, void* stream) {
     TOUED_CHECK(n_agents * n_workers > 0 && rollout_len > 0, "toued_gru_forward_tc: empty problem");
-    TOUED_CHECK(h16 != nullptr, "toued_gru_forward_tc: h16 is required");
+    // h16 is read only by the reverse pass, which also needs fac / hpimg: inference may pass NULL for all three
+    TOUED_CHECK(h16 != nullptr || (fac == nullptr && hpimg == nullptr), "toued_gru_forward_tc: h16 is required with fac / hpimg");
     return gru_forward_tc_launch(x, done, lpg_params, wh_img, h16, fac, hpimg, pi_hat, y_hat, n_agents, n_workers, rollout_len,
                                  lifetime_conditioning, 0, stream);
 }

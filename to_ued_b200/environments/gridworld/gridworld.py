@@ -229,6 +229,19 @@ class GridWorld:
                   _lib.ptr(rew), _lib.ptr(done), n, w, self.max_grid_size, self.max_n_objs, _lib.stream_ptr())
         return obs, EnvState(st, self.max_n_objs), rew, done.bool(), {}
 
+    def optimal_return(self, levels, max_rollout_len: int) -> torch.Tensor:
+        """Reference gridworld.py:253-323, batched: the optimal expected undiscounted first-episode return of every
+        level over ``max_rollout_len`` steps (each level's ``max_steps_in_episode`` caps its episode), an upper bound
+        on what any policy's evaluation (``eval_agent`` with the same horizon) can reach in expectation.  ``levels``:
+        ``EnvParams`` or packed device records ``[N, 192]``.  Returns a device f64 tensor ``[N]`` (the exact DP of
+        csrc/optimal_return.cu; no host synchronisation)."""
+        lv = self._levels(levels)
+        n = lv.shape[0]
+        out = torch.empty(n, dtype=torch.float64, device=lv.device)
+        _lib.call("toued_optimal_return", _lib.ptr(lv), n, int(max_rollout_len), self.max_grid_size, self.max_n_objs,
+                  _lib.ptr(out), _lib.stream_ptr())
+        return out
+
     def dense_obs(self, obs: torch.Tensor) -> torch.Tensor:
         """packed obs -> the reference's f32[..., D] observation (gridworld.py:184-199)."""
         idx = (obs & 0xFFFF).long()
