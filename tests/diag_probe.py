@@ -2,9 +2,10 @@
 
     TOUED_LIB_VARIANT=<variant> python tests/diag_probe.py [--poison nan|big|rand] [n_agents]
 
-Used with the library variants of csrc/build.py::VARIANTS to demonstrate the x-tile write-after-read hazard of
-the round-1 forward kernel, and with --poison to show that no kernel reads uninitialised workspace memory (the
-caching allocator's free blocks are filled with a pattern before the workspaces are allocated)."""
+Used with the schedule-fuzz library variant (csrc/build.py::VARIANTS) to show that the warp-specialised kernels give
+bit-identical results whatever the relative progress of their warps, and with --poison to show that no kernel reads
+uninitialised workspace memory (the caching allocator's free blocks are filled with a pattern before the workspaces
+are allocated)."""
 import hashlib
 import os
 import sys

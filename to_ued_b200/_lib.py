@@ -10,7 +10,7 @@ import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 # TOUED_LIB_VARIANT selects a diagnostic build of the same sources (csrc/build.py::build(variant=...)), e.g. the
-# race-probe library used by tests/diag_nondeterminism.py; production always loads libtoued.so
+# schedule-fuzz library used by tests/test_90_full_size_gpu.py; production always loads libtoued.so
 _VARIANT = os.environ.get("TOUED_LIB_VARIANT", "")
 LIB_PATH = os.path.join(_HERE, f"libtoued_{_VARIANT}.so" if _VARIANT else "libtoued.so")
 

@@ -20,23 +20,8 @@ def _nvcc():
 
 # diagnostic variants: name -> extra -D flags; built into libtoued_<name>.so next to the production library
 VARIANTS = {
-    # delays the odd-pass epilogue warps of gru_forward_tc at pass 13 so that an x-tile write-after-read hazard
-    # (if present) fires on every step (tests/diag_nondeterminism.py)
-    "probe": ["-DTOUED_RACE_PROBE=1"],
     # random delays in front of every mbarrier wait: schedule fuzzing of the warp-specialised kernels
     "fuzz": ["-DTOUED_FUZZ=1"],
-    "fuzz_old": ["-DTOUED_FUZZ=1", "-DTOUED_XTILE_OLD=1"],
-    "bwd16": ["-DBT_EW=16"],                 # 16 epilogue warps in gru_backward_tc (measured slower, see the kernel's header)
-    # weight-gradient GEMM experiments of round 2 (wgrad_tc.cu; both correct on every parity test, both measured slower):
-    "wgpair": ["-DTOUED_WGRAD_PAIR=1"],      # cta_group::2: CTA pairs sharing M256 N256 MMAs
-    "wpprobe": ["-DTOUED_WGRAD_PAIR=1", "-DTOUED_WP_PROBE=1"],   # the same with a launch-size override for timing experiments
-    "wgk": ["-DTOUED_WGRAD_KMAJOR=1"],       # K-major operands transposed in shared memory (ldmatrix.trans / stmatrix)
-    "fwdns7": ["-DFT_NS_OVERRIDE=7"],        # gru_forward_tc with 7 instead of 6 weight stages in flight
-    "fwd1": ["-DFT_HEADS_WARP=0"],           # gru_forward_tc with the heads MMAs issued by the gate-MMA warp (round-1 arrangement)
-    "pf2": ["-DBT_PF_DEPTH=2"],              # gru_backward_tc with two chunks of saved activations in flight per thread
-    "pf": ["-DBT_L2_PREFETCH=1"],            # gru_backward_tc with an L2 bulk prefetch of the next step's saved activations (measured slower)
-    "old": ["-DTOUED_XTILE_OLD=1"],
-    "probe_old": ["-DTOUED_RACE_PROBE=1", "-DTOUED_XTILE_OLD=1"],      # the round-1 x-tile writer (set 0)
 }
 
 

@@ -23,18 +23,11 @@
 #include "../../include/toued.h"
 
 constexpr int BT_M = 128;
-// Epilogue warps: warp w owns TMEM lanes [32 (w & 3), +32) and the unit slice (w >> 2) of every 64-unit block.
-// BT_EW = 8 (two 32-unit halves, 168 registers) is the production geometry.  BT_EW = 16 (four 16-unit quarters, one K-step
-// of the A stage each; library variant "bwd16") was measured in round 2: correct, but 5.96 instead of 4.24 ms per meta-step
-// -- at 608 threads the kernel is capped at 96 registers and spills 284 B per thread in the chunk loop, and four warps per
-// TMEM quadrant queue on the same tcgen05.ld port.  More warps do not buy latency hiding here; fewer instructions would.
-#ifndef BT_EW
-#define BT_EW 8
-#endif
-constexpr int BT_NQ = BT_EW / 4;                 // unit slices per 64-unit block (2 halves or 4 quarters)
-constexpr int BT_NC = 8 / BT_NQ;                 // 8-unit chunks per thread and unit block (4 or 2)
-constexpr int BT_THREADS = (BT_EW + 3) * 32;     // epilogue warps + TMA-load warp + MMA warp + TMA-store warp
-static_assert(BT_EW == 8 || BT_EW == 16, "8 or 16 epilogue warps");
+// Epilogue warps 0..7: warp w owns TMEM lanes [32 (w & 3), +32) and the 32-unit half (w >> 2) of every 64-unit block,
+// i.e. four 8-unit chunks per thread and unit block.  Eight warps keep the kernel at 168 registers; more epilogue warps
+// lower the register cap until the chunk loop spills, and more than two warps per TMEM quadrant queue on the same
+// tcgen05.ld port (DESIGN.md section 7.0).
+constexpr int BT_THREADS = 11 * 32;              // 8 epilogue warps + TMA-load warp 8 + MMA warp 9 + TMA-store warp 10
 constexpr int BT_ACHUNK = BT_M * 128;            // 16 KB: [128 rows][64 fp16], K-major SW128
 constexpr int BT_SSTAGE = 4 * BT_ACHUNK;         // stored chunks dG_r, dG_z, dG_hn (also MMA operands), dG_an: DOUBLE-buffered over the unit blocks
 constexpr int BT_CSTAGE = 2 * BT_ACHUNK;         // cz_hi, cz_lo (MMA operands only): single buffer, released K-step by K-step
@@ -65,9 +58,6 @@ __device__ __forceinline__ uint4 ldg_stream(const __half* p) {
     asm volatile("ld.global.nc.L1::no_allocate.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "l"(p));
     return r;
 }
-#ifndef BT_PF_DEPTH
-#define BT_PF_DEPTH 1                            // chunks of saved activations in flight per thread (1 or 2)
-#endif
 __device__ __forceinline__ void unpack8h(const uint4& r, float (&v)[8]) {
     const __half2* h = reinterpret_cast<const __half2*>(&r);
 #pragma unroll
@@ -92,7 +82,7 @@ gru_backward_tc_kernel(const uint8_t* __restrict__ done, const float* __restrict
     float* sWy = swp + LPG_H;                                   // [256][8]
     float* sWi = sWy + LPG_H * LPG_Y;                           // [256 units][4]: Wi row 3 x gates (r, z, n), Wi row 4 x gate r
     float* sWi2 = sWi + LPG_H * 4;                              // [256 units][2]: Wi row 4 x gates (z, n)
-    float* sdx = sWi2 + LPG_H * 2;                              // [BT_NQ - 1][128][2]
+    float* sdx = sWi2 + LPG_H * 2;                              // [128][2]
     // k_full[ks]:  K-step ks of the current unit block is in shared memory (4 epilogue warps arrive)
     // k_empty[ks]: the MMAs of that K-step have read it (cz chunks may be overwritten; also orders the reuse of a stored buffer)
     //              AND the store warp has observed k_full[ks] of this unit block (two arrivals): no waiter on k_full can
@@ -111,7 +101,7 @@ gru_backward_tc_kernel(const uint8_t* __restrict__ done, const float* __restrict
         mbar_init(&s_empty[0], 1); mbar_init(&s_empty[1], 1); mbar_init(&q_full, 1);
         mbar_fence_init();
     }
-    if (warp == BT_EW + 1) tmem_alloc(&tmem_base_s, 512);
+    if (warp == 9) tmem_alloc(&tmem_base_s, 512);
     for (int i = tid; i < LPG_H; i += BT_THREADS) swp[i] = lpg[o.w_pi + i];
     for (int i = tid; i < LPG_H * LPG_Y; i += BT_THREADS) sWy[i] = lpg[o.W_y + i];
     for (int i = tid; i < LPG_H * 6; i += BT_THREADS) {
@@ -131,7 +121,7 @@ gru_backward_tc_kernel(const uint8_t* __restrict__ done, const float* __restrict
     const size_t R32 = ((size_t)R + 31) >> 5;                   // 32-row blocks of the RB32 layout
     const size_t tstride = R32 * 32 * LPG_H;                    // RB32 elements per timestep
 
-    if (warp == BT_EW) {
+    if (warp == 8) {
         // ===================== TMA producer: Wh^T K-step slices in (unit block, K-step, gate) order ====
         if (lane == 0) {
             uint32_t it = 0;
@@ -139,22 +129,7 @@ gru_backward_tc_kernel(const uint8_t* __restrict__ done, const float* __restrict
                 if (t + 1 == L) break;                                   // the last step issues no MMAs
                 for (int ub = 0; ub < 4; ++ub)
                     for (int kk = 0; kk < 4; ++kk) {
-                        const int ks = BT_NQ == 2 ? (((kk & 1) << 1) | (kk >> 1)) : kk;
-#if defined(BT_L2_PREFETCH)        // measured in round 2 (library variant "pf"): 4.45 instead of 4.14 ms per meta-step with it -- off
-                        // L2 prefetch of the saved activations the epilogue warps will load one step from now (gates of step
-                        // t + 1, h of step t + 2): 4 KB per plane, unit block and 32-row block, spread over the 16 iterations of a
-                        // step so that the (in-order) bulk-copy queue never holds more than 20 KB in front of the Wh slices.
-                        // ncu: the epilogue warps spent ~30 % of their time waiting for these loads to return from DRAM.
-                        {
-                            const size_t blk = (size_t)(row0 >> 5) + kk;
-                            if (blk < R32) {
-                                const size_t e0 = ((((size_t)(t + 1) * R32 + blk) * 32 + ub * 8) << 8);     // rb32_index(t + 1, R32, 32 blk, 64 ub)
-#pragma unroll
-                                for (int pl = 0; pl < 4; ++pl) bulk_prefetch_l2(fac + fac_index((size_t)(t + 1), R32, (int)(blk * 32), ub * 64, pl), 8 * 256 * 2);
-                                if (t + 2 < L) bulk_prefetch_l2(h16 + e0 + tstride, 8 * 256 * 2);
-                            }
-                        }
-#endif
+                        const int ks = ((kk & 1) << 1) | (kk >> 1);
                         for (int g = 0; g < 3; ++g, ++it) {
                             const int s = it % BT_NSB;
                             mbar_wait(&b_empty[s], ((it / BT_NSB) & 1) ^ 1);
@@ -164,7 +139,7 @@ gru_backward_tc_kernel(const uint8_t* __restrict__ done, const float* __restrict
                     }
             }
         }
-    } else if (warp == BT_EW + 1) {
+    } else if (warp == 9) {
         // ===================== MMA issuer =============================================================
         // The whole warp walks the loop (all lanes wait on the barriers); one elected lane issues (tc.cuh::elect_one).
         {
@@ -182,9 +157,8 @@ gru_backward_tc_kernel(const uint8_t* __restrict__ done, const float* __restrict
                     const uint64_t ad0 = tc_smem_desc(s_addr + (ait & 1) * BT_SSTAGE);
 #pragma unroll
                     for (int kk = 0; kk < 4; ++kk) {
-                        // K-steps in the order the epilogue completes them: with two unit halves 0, 2, 1, 3 (the halves
-                        // progress together), with four quarters 0, 1, 2, 3 (all four finish at the same time)
-                        const int ks = BT_NQ == 2 ? (((kk & 1) << 1) | (kk >> 1)) : kk;
+                        // K-steps in the order the epilogue completes them: 0, 2, 1, 3 (the two unit halves progress together)
+                        const int ks = ((kk & 1) << 1) | (kk >> 1);
                         uint32_t sg[3];
                         if (mma) {
 #pragma unroll
@@ -215,7 +189,7 @@ gru_backward_tc_kernel(const uint8_t* __restrict__ done, const float* __restrict
                 }
             }
         }
-    } else if (warp == BT_EW + 2) {
+    } else if (warp == 10) {
         // ===================== TMA store warp: dG tiles of every unit block -> token-tile image ==========
         // The SW128 chunks in smem ARE the image's 8 KB sub-tiles of the weight-gradient GEMM, so they leave as
         // full-line bulk stores.  The stored chunks are double-buffered: the stores of unit block n drain while the
@@ -230,7 +204,7 @@ gru_backward_tc_kernel(const uint8_t* __restrict__ done, const float* __restrict
                 for (int ub = 0; ub < 4; ++ub, ++ait) {
 #pragma unroll
                     for (int kk = 0; kk < 4; ++kk) {                 // in completion order
-                        const int ks = BT_NQ == 2 ? (((kk & 1) << 1) | (kk >> 1)) : kk;
+                        const int ks = ((kk & 1) << 1) | (kk >> 1);
                         mbar_wait(&k_full[ks], ait & 1);
                         mbar_arrive(&k_empty[ks]);
                     }
@@ -252,7 +226,7 @@ gru_backward_tc_kernel(const uint8_t* __restrict__ done, const float* __restrict
             bulk_wait_all();
         }
     } else {
-        // ===================== epilogue / producer-of-A warps 0 .. BT_EW-1 ==============================
+        // ===================== epilogue / producer-of-A warps 0 .. 7 ====================================
         const int q = warp & 3, hf = warp >> 2;
         const int rl = q * 32 + lane;
         const int row = row0 + rl;
@@ -272,11 +246,11 @@ gru_backward_tc_kernel(const uint8_t* __restrict__ done, const float* __restrict
         //      next timestep are issued one iteration ahead (across unit-block / timestep boundaries) ----
         struct FacLoads { uint4 r, z, n, hn, hx; };              // gates of step t, h of step t+1 (the carry h')
         // per-thread element index of (t = 0, this row, this thread's first unit); chunk (ub, c8) adds (ub * 8 + c8) * 256
-        const size_t fbase = rb32_index(0, R32, rsafe, hf * (64 / BT_NQ));
-        const __half* p_r = fac + fac_index(0, R32, rsafe, hf * (64 / BT_NQ), 0);
-        const __half* p_z = fac + fac_index(0, R32, rsafe, hf * (64 / BT_NQ), 1);
-        const __half* p_n = fac + fac_index(0, R32, rsafe, hf * (64 / BT_NQ), 2);
-        const __half* p_hn = fac + fac_index(0, R32, rsafe, hf * (64 / BT_NQ), 3);
+        const size_t fbase = rb32_index(0, R32, rsafe, hf * 32);
+        const __half* p_r = fac + fac_index(0, R32, rsafe, hf * 32, 0);
+        const __half* p_z = fac + fac_index(0, R32, rsafe, hf * 32, 1);
+        const __half* p_n = fac + fac_index(0, R32, rsafe, hf * 32, 2);
+        const __half* p_hn = fac + fac_index(0, R32, rsafe, hf * 32, 3);
         const __half* p_hx = h16 + fbase;                        // + (t + 1) * tstride at use
         const int tlast = L - 1;
         auto issue_fac = [&](int t_, int ub_, int c8_) {
@@ -303,20 +277,14 @@ gru_backward_tc_kernel(const uint8_t* __restrict__ done, const float* __restrict
             r.dn_hp = t_ + 1 < L ? done[((size_t)n_ag * L + t_) * W + w_ag] : (uint8_t)1;   // the cell at t consumed (1 - done_t) h_{t+1}
             return r;
         };
-#if BT_PF_DEPTH == 2
-        FacLoads pf0 = issue_fac(0, 0, 0), pf1 = issue_fac(0, 0, 1);
-#else
         FacLoads nxt = issue_fac(0, 0, 0);
-#endif
         RowLoads rnx = issue_row(0);
         for (int t = 0; t < L; ++t) {
             const size_t tok = (size_t)t * R + rsafe;
             // head cotangents of this row (softmax backward of y_hat), lpg.py:83-84
             float dl[8], dpi;
             const RowLoads rc = rnx;
-#if BT_PF_DEPTH != 2
             if (t + 1 < L) rnx = issue_row(t + 1);
-#endif
             {
                 const float yh[8] = {rc.y0.x, rc.y0.y, rc.y0.z, rc.y0.w, rc.y1.x, rc.y1.y, rc.y1.z, rc.y1.w};
                 const float dy[8] = {rc.d0.x, rc.d0.y, rc.d0.z, rc.d0.w, rc.d1.x, rc.d1.y, rc.d1.z, rc.d1.w};
@@ -339,28 +307,19 @@ gru_backward_tc_kernel(const uint8_t* __restrict__ done, const float* __restrict
             const uint32_t p_addr = tmem_base + ((t - 1) & 1) * 256 + ((uint32_t)(q * 32) << 16);
             float dx3 = 0.f, dx4 = 0.f;
             for (int ub = 0; ub < 4; ++ub) {
-                const int ubase = ub * 64 + hf * (64 / BT_NQ);       // first of this thread's 64 / BT_NQ units
+                const int ubase = ub * 64 + hf * 32;                 // first of this thread's 32 units
                 const uint32_t sSb = sS_u32 + (ait & 1) * BT_SSTAGE;
 #pragma unroll
-                for (int c8 = 0; c8 < BT_NC; ++c8) {
+                for (int c8 = 0; c8 < 4; ++c8) {
                     const int u0 = ubase + c8 * 8;
                     float carry[8];
                     if (t > 0) tmem_ld8(p_addr + u0, carry);
-#if BT_PF_DEPTH == 2
-                    const FacLoads cur = (c8 & 1) ? pf1 : pf0;
-                    {   // prefetch the chunk after the next (same c8 parity; past the end: a harmless reload)
-                        int t2 = t, ub2 = ub, c2 = c8 + 2;
-                        if (c2 >= BT_NC) { c2 -= BT_NC; ++ub2; if (ub2 == 4) { ub2 = 0; t2 = min(t + 1, tlast); } }
-                        if (c8 & 1) pf1 = issue_fac(t2, ub2, c2); else pf0 = issue_fac(t2, ub2, c2);
-                    }
-#else
                     const FacLoads cur = nxt;
                     {   // prefetch the next chunk (next c8, else next unit block, else next timestep; past the end: a harmless reload)
                         int t2 = t, ub2 = ub, c2 = c8 + 1;
-                        if (c2 == BT_NC) { c2 = 0; ++ub2; if (ub2 == 4) { ub2 = 0; t2 = min(t + 1, tlast); } }
+                        if (c2 == 4) { c2 = 0; ++ub2; if (ub2 == 4) { ub2 = 0; t2 = min(t + 1, tlast); } }
                         nxt = issue_fac(t2, ub2, c2);
                     }
-#endif
                     if (t > 0) tmem_ld_wait();
                     else {
 #pragma unroll
@@ -420,45 +379,41 @@ gru_backward_tc_kernel(const uint8_t* __restrict__ done, const float* __restrict
                     //   first chunk of each K-step: the MMAs of the previous unit block have read that K-step (cz chunks; the
                     //   MMAs that read this stored buffer two unit blocks ago completed before those).
                     if (c8 == 0 && ait >= 2) mbar_wait(&s_empty[ait & 1], ((ait >> 1) & 1) ^ 1);
-                    if ((c8 & 1) == 0 && ait > 0) mbar_wait(&k_empty[hf * (BT_NC / 2) + (c8 >> 1)], (ait & 1) ^ 1);
-                    const uint32_t so = sw128_offset(BT_M, rl, hf * (64 / BT_NQ) + c8 * 8);
+                    if ((c8 & 1) == 0 && ait > 0) mbar_wait(&k_empty[hf * 2 + (c8 >> 1)], (ait & 1) ^ 1);
+                    const uint32_t so = sw128_offset(BT_M, rl, hf * 32 + c8 * 8);
                     st_shared_v4(sSb + so + 0 * BT_ACHUNK, pack8h_sat(gr));
                     st_shared_v4(sSb + so + 1 * BT_ACHUNK, pack8h_sat(gz));
                     st_shared_v4(sSb + so + 2 * BT_ACHUNK, pack8h_sat(ghn));
                     st_shared_v4(sSb + so + 3 * BT_ACHUNK, pack8h_sat(gan));
                     st_shared_v4(sC_u32 + so, czh4);
                     st_shared_v4(sC_u32 + so + BT_ACHUNK, czl4);
-                    if (c8 & 1) {                                  // K-step hf * BT_NC / 2 + (c8 >> 1) of this unit block is complete
+                    if (c8 & 1) {                                  // K-step 2 hf + (c8 >> 1) of this unit block is complete
                         fence_proxy_async_smem();
                         tc_fence_before();
                         __syncwarp();
-                        if (lane == 0) mbar_arrive(&k_full[hf * (BT_NC / 2) + (c8 >> 1)]);
+                        if (lane == 0) mbar_arrive(&k_full[hf * 2 + (c8 >> 1)]);
                     }
                 }
                 ++ait;
             }
-#if BT_PF_DEPTH == 2
-            if (t + 1 < L) rnx = issue_row(t + 1);       // (a step ahead costs 19 registers the second chunk in flight needs)
-#endif
-            // d pyt / d pyt1: combine the unit slices of the row (fixed order)
+            // d pyt / d pyt1: combine the two unit halves of the row (fixed order)
             if (hf > 0) { sdx[((hf - 1) * BT_M + rl) * 2] = dx3; sdx[((hf - 1) * BT_M + rl) * 2 + 1] = dx4; }
-            asm volatile("bar.sync 1, %0;" ::"n"(BT_EW * 32) : "memory");
+            asm volatile("bar.sync 1, 256;" ::: "memory");
             if (hf == 0 && rv) {
-#pragma unroll
-                for (int h2 = 0; h2 < BT_NQ - 1; ++h2) { dx3 += sdx[(h2 * BT_M + rl) * 2]; dx4 += sdx[(h2 * BT_M + rl) * 2 + 1]; }
+                dx3 += sdx[rl * 2]; dx4 += sdx[rl * 2 + 1];
                 *reinterpret_cast<float2*>(dx + ((size_t)t * R + row) * 2) = make_float2(dx3, dx4);
             }
-            asm volatile("bar.sync 1, %0;" ::"n"(BT_EW * 32) : "memory");
+            asm volatile("bar.sync 1, 256;" ::: "memory");
         }
         if (__any_sync(0xffffffffu, !(range_max <= 65504.0f)) && lane == 0 && cotmax) atomicOr(cotmax + 1, TOUED_STATUS_FP16_RANGE);
     }
     tc_fence_before();
     __syncthreads();
-    if (warp == BT_EW + 1) tmem_dealloc(tmem_base, 512);
+    if (warp == 9) tmem_dealloc(tmem_base, 512);
 }
 
 static size_t gru_bwd_tc_smem() {
-    return 2 * BT_SSTAGE + BT_CSTAGE + BT_NSB * BT_BSLICE + BT_ICHUNK + sizeof(float) * (LPG_H + LPG_H * LPG_Y + LPG_H * 6 + BT_M * 2 * (BT_NQ - 1)) + 1024;
+    return 2 * BT_SSTAGE + BT_CSTAGE + BT_NSB * BT_BSLICE + BT_ICHUNK + sizeof(float) * (LPG_H + LPG_H * LPG_Y + LPG_H * 6 + BT_M * 2) + 1024;
 }
 
 extern "C" int toued_gru_backward_tc(const uint8_t* done, const float* lpg_params, const void* whb_img,

@@ -39,20 +39,13 @@ constexpr int FT_XN = 64;                          // x-part rows: Wi_r, Wi_z, 0
 constexpr int FT_BX = (FT_XN / 8) * 256;           // 2048 B: input part (no-swizzle K=16 block: x[0..7] incl. the bias 1)
 constexpr int FT_BSTAGE = FT_BH + FT_BX;           // 26624 B per pass image (multiple of 1024)
 constexpr int FT_AX = (FT_M / 8) * 256;            // 4096 B: x tile of the A operand
-#ifndef FT_NS_OVERRIDE
 constexpr int FT_NS = 6;                  // B stages (7 measured: see DESIGN.md section 7.0)
-#else
-constexpr int FT_NS = FT_NS_OVERRIDE;
-#endif
 constexpr int FT_THEADS = 128, FT_TTILE = 192, FT_THOLD = 256;   // tensor-memory columns: 2 x 64 gate accumulators at 0, 2 x 32 head
                                                                  // accumulators, 4 x 8 relu(h) tiles, 2 x 128 columns of hidden state
-// FT_HEADS_WARP: the heads MMAs (one K = 16 MMA per pass on the relu(h) tile) are issued by a warp of their own instead of
-// by the gate-MMA warp "a few passes behind": the gate-MMA warp is a serial resource (16 passes x ~200 uniform-datapath
-// instructions and three barrier waits per step) and the epilogue warps spend 20 % of their time waiting for its MMAs.
-#ifndef FT_HEADS_WARP
-#define FT_HEADS_WARP 1
-#endif
-constexpr int FT_THREADS = 576 + 32 * FT_HEADS_WARP;   // 2 sets of 8 epilogue warps (even / odd passes) + producer warp + MMA warp (+ heads-MMA warp)
+// The heads MMAs (one K = 16 MMA per pass on the relu(h) tile) are issued by a warp of their own, not by the gate-MMA warp:
+// the gate-MMA warp is a serial resource (16 passes x ~200 uniform-datapath instructions and three barrier waits per step)
+// and the epilogue warps spend 20 % of their time waiting for its MMAs.
+constexpr int FT_THREADS = 608;           // 2 sets of 8 epilogue warps (even / odd passes) + producer warp + MMA warp + heads-MMA warp
 
 // Wh[k][c] (fp32, c = g*256 + unit) -> fp16 pass images: image[p][kb][row = g*16 + u][128 B swizzled]
 __global__ void pack_wh_fwd_kernel(const float* __restrict__ Wh, __half* __restrict__ img, size_t lpg_stride) {
@@ -199,24 +192,8 @@ gru_forward_tc_kernel(const float* __restrict__ x, const uint8_t* __restrict__ d
         // ===================== MMA issuer ==========================================================
         // The whole warp walks the loop (all lanes wait on the barriers); one elected lane issues.
         {
-            constexpr uint32_t idesc = tc_idesc(FT_M, FT_PN, 0), idesc_x = tc_idesc(FT_M, FT_XN, 0), idesc_h = tc_idesc(FT_M, 32, 0);
-            uint32_t it = 0, hq = 0;                  // hq: next pass whose heads MMA is still to be issued
-            const uint32_t hb_addr = smem_u32(sHB);
-            // heads: (pi_hat, y logits) += relu(h_t)[:, 16 units of pass q] . W_heads[16 units][32]; the A tile is read
-            // from tensor memory (written by the epilogue warps with tcgen05.st: no shared-memory staging, no proxy
-            // fence); issued a few passes behind the gate MMAs, when the tile has certainly been written
-            auto issue_heads = [&](uint32_t q) {
-                const uint32_t sb = q & 3, p = q & 15, stp = q >> 4;      // four relu(h) tiles in flight
-                mbar_wait(&stage_full[sb], (q >> 2) & 1);
-                tc_fence_after();
-                if (elect_one()) {
-                    tc_mma_ts(tmem_base + FT_THEADS + (stp & 1) * 32, tmem_base + FT_TTILE + sb * 8, tc_smem_desc_k16(hb_addr + p * 1024),
-                              idesc_h, p != 0);
-                    tc_commit(&stage_empty[sb]);
-                    if (p == 15) tc_commit(&heads_full[stp & 1]);
-                }
-                __syncwarp();
-            };
+            constexpr uint32_t idesc = tc_idesc(FT_M, FT_PN, 0), idesc_x = tc_idesc(FT_M, FT_XN, 0);
+            uint32_t it = 0;
             int cur = 0;
             for (int t = L - 1, step = 0; t >= 0; --t, ++step) {
                 if (step > 0) { mbar_wait(&a_ready, (step - 1) & 1); } else { mbar_wait(&h0_ready, 0); }
@@ -246,25 +223,16 @@ gru_forward_tc_kernel(const float* __restrict__ x, const uint8_t* __restrict__ d
                         tc_commit(&acc_full[a]);
                     }
                     __syncwarp();
-#if !FT_HEADS_WARP
-                    while (hq + 4 <= it) issue_heads(hq++);
-#endif
                 }
-#if !FT_HEADS_WARP
-                // the step's last heads MMAs: must not wait for the next step (the epilogue warps need the tile
-                // buffers back to finish this one)
-                while (hq < it) issue_heads(hq++);
-#else
-                (void)hq; (void)issue_heads;
-#endif
                 cur ^= 1;
             }
         }
-#if FT_HEADS_WARP
     } else if (warp == 18) {
         // ===================== heads-MMA issuer: follows the relu(h) tiles as the epilogue warps publish them.  Ordering with
         // the readout of the head accumulators two steps earlier is transitive: readout(s) precedes that warp's passes of step
         // s + 1, hence a_ready(s + 1), hence the gate MMAs and relu tiles of step s + 2 this warp waits for.
+        // Per pass q: (pi_hat, y logits) += relu(h_t)[:, 16 units of pass q] . W_heads[16 units][32]; the A tile is read from
+        // tensor memory (written by the epilogue warps with tcgen05.st: no shared-memory staging, no proxy fence).
         constexpr uint32_t idesc_h = tc_idesc(FT_M, 32, 0);
         const uint32_t hb_addr = smem_u32(sHB);
         const uint32_t nq = (uint32_t)L * FT_NPASS;
@@ -280,7 +248,6 @@ gru_forward_tc_kernel(const float* __restrict__ x, const uint8_t* __restrict__ d
             }
             __syncwarp();
         }
-#endif
     } else {
         // ===================== epilogue warps: set 0 (warps 0..7) takes the even passes / accumulator 0,
         // set 1 (warps 8..15) the odd passes / accumulator 1.  A pass is one long dependent chain per warp
@@ -312,12 +279,8 @@ gru_forward_tc_kernel(const float* __restrict__ x, const uint8_t* __restrict__ d
             // set 1: only a set-1 warp has observed acc_full of that pass, i.e. knows that every MMA reading the tile
             // has completed.  (Round 1 wrote it from set 0, whose last pass is 14: when set 1 lagged by one pass the
             // MMA of pass 15 read x of the wrong time step for 16 units -- the source of the run-to-run differences
-            // of the BASELINE-size step; tests/diag_nondeterminism.py reproduces it with the probe build.)
-#if defined(TOUED_XTILE_OLD)
-            if (set == 0 && hf == 0 && t > 0) {
-#else
+            // of the BASELINE-size step.)
             if (set == 1 && hf == 0 && t > 0) {
-#endif
                 uint4 pk = make_uint4(0u, 0u, 0u, 0u);
                 if (rv) {
                     const float4* xp = reinterpret_cast<const float4*>(x + ((size_t)(t - 1) * R + row) * LPG_XP);
@@ -341,9 +304,6 @@ gru_forward_tc_kernel(const float* __restrict__ x, const uint8_t* __restrict__ d
             for (int p = set; p < FT_NPASS; p += 2) {
                 const uint32_t it = (uint32_t)step * FT_NPASS + p;
                 const int a = set;
-#if defined(TOUED_RACE_PROBE)
-                if (set == 1 && p == 13) __nanosleep(20000);      // diagnostic build: let set 0 run a full pass ahead
-#endif
                 mbar_wait(&acc_full[a], (it >> 1) & 1);
                 tc_fence_after();
                 float ar[8], az[8], an[8], ai[8];

@@ -7,7 +7,6 @@
 // output tile (fp32 accumulators in 384 TMEM columns) and a contiguous range of token blocks; the four
 // tile types of one token range are adjacent CTAs so they share their operand stream through L2.
 // Output: per-split partial sums (deterministic; reduced by toued_reduce_partials).
-#include <cstdlib>
 #include "tc.cuh"
 #include "lpg_common.cuh"
 #include "../../include/toued.h"
@@ -467,376 +466,7 @@ wgrad_heads_mma_kernel(const __half* __restrict__ h16, const float* __restrict__
     if (warp == 5) tmem_dealloc(tmem_base, 64);
 }
 
-// ------------------------------------------------------------------------------------------------
-// CTA-PAIR version of the weight-gradient GEMMs (round 2; library variant "wgpair", NOT the default -- measured slower).
-// The 1-CTA kernel above is operand-bound: two M128 N192 MMAs per K-step take 509 clk for 192 clk of math (tensor pipe
-// 67 % active in ncu).  With cta_group::2 a pair of CTAs shares M256 MMAs: each CTA holds its own 128 rows of A and HALF
-// of B's N columns, i.e. it reads 4 + 4 KB of shared memory per M256 N256 K16 MMA for 128 clk of math.
-// MEASURED (B200, one pair alone on the GPU, 366 token blocks): 376 clk per M256 N256 K16 MMA -- 1,394 MAC per SM-clock
-// against 1,547 for the 1-CTA kernel.  The bound is therefore not the shared-memory bytes per CTA: both kernels ingest
-// MN-major (token-contracted) operands at ~20 elements per clock, 2.7 - 2.9 x the math time, whichever way the tile is
-// split.  Whole launch: 330 us (pair) against 208 us (1-CTA).  The kernel is correct (every tensor-core parity test passes
-// with it) and stays as the worked example of the cta_group::2 protocol on this code base.
-//   * dWh pair tiles: M = 256 hidden units j (CTA r: its 128), N = 256 gate columns c of gate ct (CTA r: 128 of them),
-//     K = tokens: one MMA per K-step, 32 KB of operands per 64-token block and CTA, ring of 6 stages.
-//   * input-side pair tiles (dWi, db_i, db_hn): roles swapped -- M = 256 of the 1024 dG columns per MMA (four MMAs per
-//     K-step), N = the x column group (each CTA supplies the same 64 columns; only the first 8 are inputs), so the wide
-//     dG operand is the 128-row A side: 72 KB per 64-token block and CTA, ring of 3.
-// Pairs [0, 3 S1) are dWh tiles (gate ct = pair % 3, token split pair / 3), pairs [3 S1, 3 S1 + S2) input-side tiles; the
-// input-side tiles stream 2.25 x the operands per token block, hence their own (larger) split count.
-// The follower CTA's bulk copies complete on its own mbarrier; one of its threads relays each completion to the leader
-// (remote arrive), the leader's commits release the stage in both CTAs (multicast).
-constexpr int WP_THREADS = 192;            // 4 epilogue warps + producer warp + MMA (leader) / relay (follower) warp
-constexpr int WP_SMEM = 216 * 1024;
-constexpr int WP_S1 = 14, WP_S2 = 32;      // 3 * 14 + 32 = 74 pairs = 148 CTAs
-static_assert(WP_S1 <= 37 && WP_S2 <= 148, "partial areas (lpg_backward.cu / wgrad_heads) are sized for 37 / 148 splits");
-
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(WP_THREADS, 1)
-wgrad_pair_kernel(const unsigned char* __restrict__ hpimg, const unsigned char* __restrict__ dgimg,
-                  const unsigned char* __restrict__ ximg, float* __restrict__ partial, float* __restrict__ small_partial,
-                  const uint32_t* __restrict__ cotmax, int n_tok_blocks, int bps_wh, int bps_x, int accumulate) {
-    extern __shared__ __align__(1024) unsigned char smem_raw[];
-    unsigned char* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
-    __shared__ __align__(8) uint64_t full[6], peer_full[6], empty[6], done_bar;
-    __shared__ uint32_t tmem_base_s;
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const uint32_t rank = cluster_ctarank();
-    const int pair = blockIdx.x >> 1;
-    const bool xt = pair >= 3 * WP_S1;
-    const int ct = pair % 3;
-    const int split = xt ? pair - 3 * WP_S1 : pair / 3;
-    const int bps = xt ? bps_x : bps_wh;
-    const int NS = xt ? 3 : 6;
-    const uint32_t STAGE = xt ? 9 * 8192 : 4 * 8192;
-    const int tb0 = split * bps;
-    const int nblk = max(0, min(n_tok_blocks, tb0 + bps) - tb0);
-
-    if (tid == 0) {
-        for (int s = 0; s < 6; ++s) { mbar_init(&full[s], 1); mbar_init(&peer_full[s], 1); mbar_init(&empty[s], 1); }
-        mbar_init(&done_bar, 1);
-        mbar_fence_init();
-    }
-    if (warp == 5) tmem_alloc2(&tmem_base_s, 512);
-    tc_fence_before();
-    __syncthreads();
-    cluster_sync();                            // both CTAs' barriers exist before any remote / multicast arrival
-    tc_fence_after();
-    const uint32_t tmem_base = tmem_base_s;
-
-    if (warp == 4) {
-        // ---- producer: this CTA's halves of the operands ----
-        if (lane == 0) {
-            for (int i = 0; i < nblk; ++i) {
-                const int s = i % NS;
-                mbar_wait_cluster(&empty[s], ((i / NS) & 1) ^ 1);
-                mbar_expect_tx(&full[s], STAGE);
-                unsigned char* st = smem + s * STAGE;
-                const size_t tb = (size_t)(tb0 + i);
-                if (!xt) {
-                    bulk_g2s(st, hpimg + ((tb * 4 + 2 * rank) << 13), 2 * 8192, &full[s]);                    // j groups 2r, 2r+1
-                    bulk_g2s(st + 2 * 8192, dgimg + ((tb * 16 + 4 * ct + 2 * rank) << 13), 2 * 8192, &full[s]); // c groups of gate ct
-                } else {
-#pragma unroll
-                    for (int m = 0; m < 4; ++m)                                                                  // dG groups 4m + 2r, + 1
-                        bulk_g2s(st + m * 2 * 8192, dgimg + ((tb * 16 + 4 * m + 2 * rank) << 13), 2 * 8192, &full[s]);
-                    bulk_g2s(st + 8 * 8192, ximg + (tb << 13), 8192, &full[s]);                                  // the x group
-                }
-            }
-        }
-    } else if (warp == 5) {
-        if (rank != 0) {
-            // ---- follower: relay "my operands have landed" to the leader ----
-            if (lane == 0)
-                for (int i = 0; i < nblk; ++i) {
-                    const int s = i % NS;
-                    mbar_wait(&full[s], (i / NS) & 1);
-                    mbar_arrive_remote(&peer_full[s], 0);
-                }
-        } else {
-            // ---- leader: MMA issue for the pair (all lanes wait, one elected lane issues) ----
-            constexpr uint32_t idesc_wh = tc_idesc_mn(256, 256, 0), idesc_x = tc_idesc_mn(256, 128, 0);      // fp16
-            for (int i = 0; i < nblk; ++i) {
-                const int s = i % NS;
-                mbar_wait(&full[s], (i / NS) & 1);
-                mbar_wait_cluster(&peer_full[s], (i / NS) & 1);
-                tc_fence_after();
-                const uint32_t a0 = smem_u32(smem + s * STAGE);
-                if (elect_one()) {
-                    if (!xt) {
-#pragma unroll
-                        for (int ks = 0; ks < 4; ++ks)
-                            tc_mma2(tmem_base, tc_smem_desc_mn(a0 + ks * 2048, 8192), tc_smem_desc_mn(a0 + 2 * 8192 + ks * 2048, 8192),
-                                    idesc_wh, (i | ks) != 0);
-                    } else {
-#pragma unroll
-                        for (int ks = 0; ks < 4; ++ks)
-#pragma unroll
-                            for (int m = 0; m < 4; ++m)
-                                tc_mma2(tmem_base + m * 128, tc_smem_desc_mn(a0 + m * 2 * 8192 + ks * 2048, 8192),
-                                        tc_smem_desc_mn(a0 + 8 * 8192 + ks * 2048, 8192), idesc_x, (i | ks) != 0);
-                    }
-                    tc_commit2(&empty[s], 3);
-                }
-                __syncwarp();
-            }
-            if (elect_one()) tc_commit2(&done_bar, 3);
-            __syncwarp();
-        }
-    } else {
-        // ---- epilogue (both CTAs): TMEM lane = this CTA's row of the M = 256 tile ----
-        mbar_wait_cluster(&done_bar, 0);
-        tc_fence_after();
-        // the dG image is in units of the launch's cotangent scale S (tc.cuh): take it back out of the fp32 sums
-        const float inv_s = cotmax ? 1.0f / cot_scale_from_max(*cotmax) : 1.0f;
-        const uint32_t trow = tmem_base + ((uint32_t)(warp * 32) << 16);
-        if (!xt) {
-            const int j = (int)rank * 128 + warp * 32 + lane;
-            float* out = partial + (size_t)split * LPG_H * LPG_G + (size_t)j * LPG_G + ct * 256;
-            // 64 columns per round: the previous partials are fetched with 16 independent loads in flight
-            for (int c = 0; c < 256; c += 64) {
-                float4 pre[16];
-                float4* p = reinterpret_cast<float4*>(out + c);
-                if (accumulate) {
-#pragma unroll
-                    for (int i = 0; i < 16; ++i) pre[i] = p[i];
-                } else {
-#pragma unroll
-                    for (int i = 0; i < 16; ++i) pre[i] = make_float4(0.f, 0.f, 0.f, 0.f);
-                }
-#pragma unroll
-                for (int i = 0; i < 8; ++i) {
-                    float v[8];
-                    if (nblk > 0) {
-                        tmem_ld8(trow + c + 8 * i, v);
-                        tmem_ld_wait();
-                    } else {
-#pragma unroll
-                        for (int e = 0; e < 8; ++e) v[e] = 0.f;
-                    }
-                    p[2 * i] = make_float4(fmaf(v[0], inv_s, pre[2 * i].x), fmaf(v[1], inv_s, pre[2 * i].y), fmaf(v[2], inv_s, pre[2 * i].z), fmaf(v[3], inv_s, pre[2 * i].w));
-                    p[2 * i + 1] = make_float4(fmaf(v[4], inv_s, pre[2 * i + 1].x), fmaf(v[5], inv_s, pre[2 * i + 1].y), fmaf(v[6], inv_s, pre[2 * i + 1].z), fmaf(v[7], inv_s, pre[2 * i + 1].w));
-                }
-            }
-        } else if (nblk > 0) {
-            // rows = dG columns: chunk m holds c = 256 m + 128 rank + row; columns 0..7 = the x inputs q (7 = the bias 1).
-            // Always accumulates: the head-gradient kernel has initialised this split's small-partial area.
-            float* out = small_partial + (size_t)split * SMT_TOTAL;
-            const int cl = (int)rank * 128 + warp * 32 + lane;            // column within the gate block
-#pragma unroll
-            for (int m = 0; m < 4; ++m) {
-                float v[8];
-                tmem_ld8(trow + m * 128, v);
-                tmem_ld_wait();
-                if (m == 2) {
-                    out[SMT_BHN + cl] = fmaf(v[7], inv_s, out[SMT_BHN + cl]);                  // sum of dhn = d b_hn
-                } else {
-                    const int col = (m == 3 ? 512 : m * 256) + cl;                             // dar | daz | dan columns of W_i
-#pragma unroll
-                    for (int q = 0; q < 8; ++q) out[SMT_WI + q * LPG_G + col] = fmaf(v[q], inv_s, out[SMT_WI + q * LPG_G + col]);
-                }
-            }
-        }
-    }
-    tc_fence_before();
-    __syncthreads();
-    cluster_sync();                            // nobody releases tensor memory while the peer may still use the pair
-    if (warp == 5) tmem_dealloc2(tmem_base, 512);
-}
-
-// ------------------------------------------------------------------------------------------------
-// TRANSPOSING version of the weight-gradient GEMMs (round 2; library variant "wgk", NOT the default -- measured slower:
-// 408 us per launch against 208 us.  Correct on every tensor-core parity test.  Per 64-token block a CTA moves 40 KB four
-// times through shared memory -- bulk-copy write, ldmatrix read, stmatrix write, tensor-core read = 160 KB, ~1,250 clk at
-// 128 B/clk, measured 1,877 clk -- which costs more than the MN-major ingestion it was meant to avoid.)
-// The MMAs of the kernels above take their
-// operands MN-major (contraction over tokens = rows of the token tile images) and run at 2.7 x their math time: the
-// tensor core ingests MN-major operands at ~20 elements per clock, whichever way the tile is cut (measured with the
-// CTA-pair kernel).  K-major operands stream at the math rate (gru_backward_tc: M128 N256 K16 in ~108 clk).  So this
-// kernel turns every 64-token x 64-column sub-tile around in shared memory before the MMA reads it:
-//   producer warp     bulk copies of the raw sub-tiles (as they lie in the images) into a 2-stage ring;
-//   4 transposer warps  ldmatrix.x4.trans + stmatrix.x4: four 8 x 8 blocks per instruction pair, raw [token][column] SW128 ->
-//                     K-major [column][token] SW128 tiles (2-stage ring), then fence.proxy.async + mbarrier;
-//   MMA warp          per 64-token block four K = 16 MMAs on K-major descriptors; commits release the K-major stage;
-//   the transposer warps are also the epilogue warps (TMEM -> partial sums, as above).
-// 12 tile types of equal cost (5 sub-tiles = 40 KB per token block): 8 dWh tiles (128 hidden units j x 192 gate columns c)
-// and 4 input-side tiles (the x group, M = 64, x 256 of the 1024 dG columns), 12 token splits each = 144 CTAs.
-constexpr int WK_THREADS = 192;            // 4 transposer / epilogue warps + producer warp + MMA warp
-constexpr int WK_SPLITS = 12;
-constexpr int WK_STAGE = 5 * 8192;         // 5 sub-tiles: A (2 for dWh: j groups; 1 for x) + B (3 for dWh; 4 for x)
-static_assert(WK_SPLITS <= 37, "Wh partial areas (lpg_backward.cu) are sized for 37 splits");
-
-__device__ __forceinline__ void ldsm_x4_trans(uint32_t addr, uint32_t (&r)[4]) {
-    asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0, %1, %2, %3}, [%4];"
-                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]) : "r"(addr));
-}
-__device__ __forceinline__ void stsm_x4(uint32_t addr, const uint32_t (&r)[4]) {
-    asm volatile("stmatrix.sync.aligned.m8n8.x4.shared.b16 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]) : "memory");
-}
-
-__global__ void __launch_bounds__(WK_THREADS, 1)
-wgrad_kmajor_kernel(const unsigned char* __restrict__ hpimg, const unsigned char* __restrict__ dgimg,
-                    const unsigned char* __restrict__ ximg, float* __restrict__ partial, float* __restrict__ small_partial,
-                    const uint32_t* __restrict__ cotmax, int n_tok_blocks, int blocks_per_split, int accumulate) {
-    extern __shared__ __align__(1024) unsigned char smem_raw[];
-    unsigned char* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
-    unsigned char* sRaw = smem;                             // 2 x 40 KB   raw sub-tiles [token][column]
-    unsigned char* sK = smem + 2 * WK_STAGE;                // 2 x 40 KB   K-major tiles [column][token]
-    __shared__ __align__(8) uint64_t raw_full[2], raw_empty[2], k_full[2], k_empty[2], done_bar;
-    __shared__ uint32_t tmem_base_s;
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    // types 0-7: dWh tile (jt, cq): h'^T [128 j] x dG columns [192 cq, 192 cq + 192);  types 8-11: x^T x dG columns [256 xq, +256)
-    const int type = blockIdx.x % 12, split = blockIdx.x / 12;
-    const bool xt = type >= 8;
-    const int jt = type >> 2, cq = type & 3, xq = type - 8;
-    const int tb0 = split * blocks_per_split;
-    const int nblk = max(0, min(n_tok_blocks, tb0 + blocks_per_split) - tb0);
-
-    if (tid == 0) {
-        for (int s = 0; s < 2; ++s) {
-            mbar_init(&raw_full[s], 1); mbar_init(&raw_empty[s], 4); mbar_init(&k_full[s], 4); mbar_init(&k_empty[s], 1);
-        }
-        mbar_init(&done_bar, 1);
-        mbar_fence_init();
-    }
-    if (warp == 5) tmem_alloc(&tmem_base_s, 256);
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = tmem_base_s;
-
-    if (warp == 4) {
-        // ---- producer: raw sub-tiles.  Stage layout: dWh [A j-group 0 | A j-group 1 | B 3 column groups]; x [A x group | B 4 groups]
-        if (lane == 0) {
-            for (int i = 0; i < nblk; ++i) {
-                const int s = i & 1;
-                mbar_wait(&raw_empty[s], ((i >> 1) & 1) ^ 1);
-                mbar_expect_tx(&raw_full[s], WK_STAGE);
-                unsigned char* st = sRaw + s * WK_STAGE;
-                const size_t tb = (size_t)(tb0 + i);
-                if (!xt) {
-                    bulk_g2s(st, hpimg + ((tb * 4 + 2 * jt) << 13), 2 * 8192, &raw_full[s]);
-                    bulk_g2s(st + 2 * 8192, dgimg + ((tb * 16 + 3 * cq) << 13), 3 * 8192, &raw_full[s]);
-                } else {
-                    bulk_g2s(st, ximg + (tb << 13), 8192, &raw_full[s]);
-                    bulk_g2s(st + 8192, dgimg + ((tb * 16 + 4 * xq) << 13), 4 * 8192, &raw_full[s]);
-                }
-            }
-        }
-    } else if (warp == 5) {
-        // ---- MMA issue on the K-major tiles (all lanes wait, one elected lane issues)
-        constexpr uint32_t idesc_wh = tc_idesc(128, 192, 0), idesc_x = tc_idesc(64, 256, 0);       // fp16, both operands K-major
-        for (int i = 0; i < nblk; ++i) {
-            const int s = i & 1;
-            mbar_wait(&k_full[s], (i >> 1) & 1);
-            tc_fence_after();
-            const uint32_t k0 = smem_u32(sK + s * WK_STAGE);
-            if (elect_one()) {
-                const uint64_t ad = tc_smem_desc(k0), bd = tc_smem_desc(k0 + (xt ? 8192 : 2 * 8192));
-#pragma unroll
-                for (int ks = 0; ks < 4; ++ks)                      // K = 16 tokens = 32 B along the 128-byte token rows
-                    tc_mma(tmem_base, ad + 2 * ks, bd + 2 * ks, xt ? idesc_x : idesc_wh, (i | ks) != 0);
-                tc_commit(&k_empty[s]);
-            }
-            __syncwarp();
-        }
-        if (elect_one()) tc_commit(&done_bar);
-        __syncwarp();
-    } else {
-        // ---- transposer warps: 5 sub-tiles x 16 groups of four 8 x 8 blocks, 20 groups per warp and token block
-        const int mi = lane >> 3, ri = lane & 7;
-        for (int i = 0; i < nblk; ++i) {
-            const int s = i & 1;
-            mbar_wait(&raw_full[s], (i >> 1) & 1);
-            mbar_wait(&k_empty[s], ((i >> 1) & 1) ^ 1);
-            const uint32_t src0 = smem_u32(sRaw + s * WK_STAGE), dst0 = smem_u32(sK + s * WK_STAGE);
-#pragma unroll 4
-            for (int g = warp; g < 80; g += 4) {
-                const int sub = g >> 4, gg = g & 15;
-                const int tc8 = gg >> 1, cc = (gg & 1) * 4 + mi;      // token chunk, column chunk of this lane's block
-                // source block: rows = tokens tc8*8 + ri, 16-byte chunk cc (swizzled by the row)
-                const uint32_t sa = src0 + sub * 8192 + (tc8 * 8 + ri) * 128 + ((cc ^ ri) << 4);
-                // destination block: rows = columns cc*8 + ri of the sub-tile, 16-byte chunk tc8 (swizzled by the row)
-                const uint32_t da = dst0 + sub * 8192 + (cc * 8 + ri) * 128 + ((tc8 ^ ri) << 4);
-                uint32_t r[4];
-                ldsm_x4_trans(sa, r);
-                stsm_x4(da, r);
-            }
-            fence_proxy_async_smem();                                 // generic-proxy stores -> tensor-core (async proxy) reads
-            __syncwarp();
-            if (lane == 0) { mbar_arrive(&raw_empty[s]); mbar_arrive(&k_full[s]); }
-        }
-        // ---- epilogue: TMEM lane = row of the tile
-        mbar_wait(&done_bar, 0);
-        tc_fence_after();
-        // the dG image is in units of the launch's cotangent scale S (tc.cuh): take it back out of the fp32 sums
-        const float inv_s = cotmax ? 1.0f / cot_scale_from_max(*cotmax) : 1.0f;
-        if (xt) {
-            // rows 0..7 of the x tile: dWi (rows q < X), dbi (row 7) and dbhn (row 7 of the dhn columns).
-            // Always accumulates: the head-gradient kernel has initialised this split's small-partial area.
-            if (warp == 0 && nblk > 0) {
-                float* out = small_partial + (size_t)split * SMT_TOTAL;
-                const int base = xq == 3 ? SMT_WI + lane * LPG_G + 512 : (xq == 2 ? SMT_BHN : SMT_WI + lane * LPG_G + 256 * xq);
-                const bool on = lane < 8 && (xq != 2 || lane == 7);
-                for (int c = 0; c < 256; c += 32) {          // 32 columns per round: loads first, then the stores
-                    float v[4][8], o[4][8];
-#pragma unroll
-                    for (int k = 0; k < 4; ++k) tmem_ld8(tmem_base + c + 8 * k, v[k]);
-                    tmem_ld_wait();
-                    if (on) {
-#pragma unroll
-                        for (int k = 0; k < 4; ++k)
-#pragma unroll
-                            for (int e = 0; e < 8; ++e) o[k][e] = out[base + c + 8 * k + e];
-#pragma unroll
-                        for (int k = 0; k < 4; ++k)
-#pragma unroll
-                            for (int e = 0; e < 8; ++e) out[base + c + 8 * k + e] = fmaf(v[k][e], inv_s, o[k][e]);
-                    }
-                }
-            }
-        } else {
-            const int j = jt * 128 + warp * 32 + lane;
-            float* out = partial + (size_t)split * LPG_H * LPG_G + (size_t)j * LPG_G + cq * 192;
-            // 64 columns per round: the previous partials are fetched with 16 independent loads in flight
-            for (int c = 0; c < 192; c += 64) {
-                float4 pre[16];
-                float4* p = reinterpret_cast<float4*>(out + c);
-                if (accumulate) {
-#pragma unroll
-                    for (int k = 0; k < 16; ++k) pre[k] = p[k];
-                } else {
-#pragma unroll
-                    for (int k = 0; k < 16; ++k) pre[k] = make_float4(0.f, 0.f, 0.f, 0.f);
-                }
-#pragma unroll
-                for (int k = 0; k < 8; ++k) {
-                    float v[8];
-                    if (nblk > 0) {
-                        tmem_ld8(tmem_base + ((uint32_t)(warp * 32) << 16) + c + 8 * k, v);
-                        tmem_ld_wait();
-                    } else {
-#pragma unroll
-                        for (int e = 0; e < 8; ++e) v[e] = 0.f;
-                    }
-                    p[2 * k] = make_float4(fmaf(v[0], inv_s, pre[2 * k].x), fmaf(v[1], inv_s, pre[2 * k].y), fmaf(v[2], inv_s, pre[2 * k].z), fmaf(v[3], inv_s, pre[2 * k].w));
-                    p[2 * k + 1] = make_float4(fmaf(v[4], inv_s, pre[2 * k + 1].x), fmaf(v[5], inv_s, pre[2 * k + 1].y), fmaf(v[6], inv_s, pre[2 * k + 1].z), fmaf(v[7], inv_s, pre[2 * k + 1].w));
-                }
-            }
-        }
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 5) tmem_dealloc(tmem_base, 256);
-}
-
-#if defined(TOUED_WGRAD_KMAJOR)
-constexpr int WT_SPLITS = WK_SPLITS;       // 12 tile types x 12 = 144 CTAs
-#elif !defined(TOUED_WGRAD_PAIR)
 constexpr int WT_SPLITS = 24;              // 6 tile types x 24 = 144 CTAs
-#else
-constexpr int WT_SPLITS = WP_S1;           // dWh partial areas written by the pair kernel
-#endif
-
 static_assert(WT_SPLITS <= 37 && HT_SPLITS <= 592, "partial areas of toued_lpg_wgrad_workspace_floats (lpg_backward.cu) are sized for 37 / 592 splits");
 extern "C" int toued_wgrad_tc_splits(void) { return WT_SPLITS; }
 extern "C" int toued_wgrad_tc_small_splits(void) { return HT_SPLITS; }
@@ -866,30 +496,11 @@ extern "C" int toued_lpg_wgrad_tc(const void* hpimg, const void* dgimg, const vo
                                                                          cotangent_max, R, L, rbps, accumulate);
     }
     TOUED_LAUNCH_CHECK();
-#if defined(TOUED_WGRAD_KMAJOR)
-    const size_t smem = 4 * WK_STAGE + 1024;
-    TOUED_CUDA(cudaFuncSetAttribute(wgrad_kmajor_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    wgrad_kmajor_kernel<<<12 * WK_SPLITS, WK_THREADS, smem, st>>>((const unsigned char*)hpimg, (const unsigned char*)dgimg,
-                                                                  (const unsigned char*)ximg, wh_partials, small_partials,
-                                                                  cotangent_max, n_tb, bps, accumulate);
-#elif !defined(TOUED_WGRAD_PAIR)
     const size_t smem = WT_NS * WT_STAGE + 1024;
     TOUED_CUDA(cudaFuncSetAttribute(wgrad_wh_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     wgrad_wh_tc_kernel<<<6 * WT_SPLITS, WT_THREADS, smem, st>>>((const unsigned char*)hpimg, (const unsigned char*)dgimg,
                                                                 (const unsigned char*)ximg, wh_partials, small_partials,
                                                                 cotangent_max, n_tb, bps, accumulate);
-#else
-    (void)bps;
-    const size_t smem = WP_SMEM + 1024;
-    TOUED_CUDA(cudaFuncSetAttribute(wgrad_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int npairs = 3 * WP_S1 + WP_S2;
-#if defined(TOUED_WP_PROBE)      // timing experiments only (results are incomplete): launch just the first N pairs
-    if (const char* e = getenv("TOUED_WP_PAIRS")) npairs = atoi(e);
-#endif
-    wgrad_pair_kernel<<<2 * npairs, WP_THREADS, smem, st>>>(
-        (const unsigned char*)hpimg, (const unsigned char*)dgimg, (const unsigned char*)ximg, wh_partials, small_partials,
-        cotangent_max, n_tb, (n_tb + WP_S1 - 1) / WP_S1, (n_tb + WP_S2 - 1) / WP_S2, accumulate);
-#endif
     TOUED_LAUNCH_CHECK();
     return 0;
 }
