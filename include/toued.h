@@ -296,6 +296,10 @@ int toued_tc_gemm_mn_test(const float* A, const float* B, void* scratch_img, flo
 /* the same contraction on a CTA pair (cta_group::2, M = 256 over a 2-cluster): D f32[256][256] = A[128 k][256 m]^T B[128 k][256 n];
  * scratch_img >= 128 KiB                                                                              */
 int toued_tc_gemm_mn2_test(const float* A, const float* B, void* scratch_img, float* D, void* stream);
+/* the weight-gradient GEMM's operand roles, fp16 (csrc/wgrad_tc.cu): D f32[128][256 + 16] = A[128 k][128 m]^T [B[128 k][256 n] |
+ * X[128 k][0:16]] with X f32[128 k][64]; the X operand is the first 16 columns of one 64-column SW128 group (N = 16).
+ * scratch_img >= 112 KiB                                                                              */
+int toued_tc_gemm_mn_x16_test(const float* A, const float* B, const float* X, void* scratch_img, float* D, void* stream);
 
 /* Pack the recurrent matrix Wh (+ input projection Wi, b_i) into the fp16 pass images the tensor-core
  * forward streams (wh_img: 16 x 26 KiB = 416 KiB, once per meta-step).                              */

@@ -83,6 +83,7 @@ SIGNATURES = {
     "toued_tc_gemm_mixed_test": [_P] * 5,
     "toued_tc_gemm_mn_test": [_P] * 4 + [_I] * 3 + [_P],
     "toued_tc_gemm_mn2_test": [_P] * 5,
+    "toued_tc_gemm_mn_x16_test": [_P] * 6,
     "toued_pack_wh_forward": [_P, _P, _I, _P],
     "toued_pack_wh_forward_multi": [_P, _P, _I, _I, _I, _P],
     "toued_gru_forward_tc_multi": [_P] * 6 + [_I] * 5 + [_P],

@@ -304,3 +304,79 @@ extern "C" int toued_tc_gemm_mixed_test(const float* A, const float* B, void* sc
     TOUED_LAUNCH_CHECK();
     return 0;
 }
+
+// ------------------------------------------------------------------------------------------------
+// The weight-gradient GEMM's operand roles (wgrad_tc.cu), fp16, K = 128 tokens: one MN-major A of 128 columns
+// (two 64-column groups) against (a) B = 256 columns (four groups, N = 256) and (b) B = the first 16 columns of a
+// single 64-column group (N = 16: an MN-major SW128 operand narrower than its 64-element swizzle atom, as the x image
+// is used).  D[128][256 + 16] = A^T [B | X[:, 0:16]].
+__global__ void pack_tile_img_f16_kernel(const float* __restrict__ X, __half* __restrict__ img, int K, int C) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= K * C) return;
+    const int k = i / C, c = i % C;
+    *reinterpret_cast<__half*>(reinterpret_cast<char*>(img) + tile_img_offset(k, C / 64, c)) = __float2half_rn(X[i]);
+}
+
+__global__ void __launch_bounds__(128, 1)
+tc_gemm_mn_x16_test_kernel(const unsigned char* __restrict__ Aimg, const unsigned char* __restrict__ Bimg,
+                           const unsigned char* __restrict__ Ximg, float* __restrict__ D) {
+    extern __shared__ __align__(1024) unsigned char smem_raw[];
+    unsigned char* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
+    unsigned char* sA = smem;               // 2 token blocks x [2 col groups][8 KB]
+    unsigned char* sB = smem + 32768;       // 2 token blocks x [4 col groups][8 KB]
+    unsigned char* sX = smem + 98304;       // 2 token blocks x [1 col group][8 KB]
+    __shared__ __align__(8) uint64_t bar_ld, bar_mma;
+    __shared__ uint32_t tmem_base;
+    const int tid = threadIdx.x, warp = tid >> 5;
+    if (warp == 0) tmem_alloc(&tmem_base, 512);
+    if (tid == 0) { mbar_init(&bar_ld, 1); mbar_init(&bar_mma, 1); mbar_fence_init(); }
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+    const uint32_t tb = tmem_base;
+    if (tid == 0) {
+        mbar_expect_tx(&bar_ld, 32768 + 65536 + 16384);
+        bulk_g2s(sA, Aimg, 32768, &bar_ld);
+        bulk_g2s(sB, Bimg, 65536, &bar_ld);
+        bulk_g2s(sX, Ximg, 16384, &bar_ld);
+        mbar_wait(&bar_ld, 0);
+        tc_fence_after();
+        constexpr uint32_t idesc = tc_idesc_mn(128, 256, 0), idesc_x = tc_idesc_mn(128, 16, 0);
+        for (int blk = 0; blk < 2; ++blk)
+            for (int ks = 0; ks < 4; ++ks) {
+                const uint64_t ad = tc_smem_desc_mn(smem_u32(sA + blk * 16384 + ks * 2048), 8192);
+                tc_mma(tb, ad, tc_smem_desc_mn(smem_u32(sB + blk * 32768 + ks * 2048), 8192), idesc, (blk | ks) != 0);
+                tc_mma(tb + 256, ad, tc_smem_desc_mn(smem_u32(sX + blk * 8192 + ks * 2048), 8192), idesc_x, (blk | ks) != 0);
+            }
+        tc_commit(&bar_mma);
+    }
+    mbar_wait(&bar_mma, 0);
+    tc_fence_after();
+    for (int c = 0; c < 272; c += 8) {
+        float v[8];
+        tmem_ld8(tb + ((uint32_t)(warp * 32) << 16) + c, v);
+        tmem_ld_wait();
+#pragma unroll
+        for (int e = 0; e < 8; ++e) D[tid * 272 + c + e] = v[e];
+    }
+    tc_fence_before();
+    __syncthreads();
+    if (warp == 0) tmem_dealloc(tb, 512);
+}
+
+extern "C" int toued_tc_gemm_mn_x16_test(const float* A, const float* B, const float* X, void* scratch_img, float* D,
+                                         void* stream) {
+    cudaStream_t st = (cudaStream_t)stream;
+    unsigned char* ia = (unsigned char*)scratch_img;
+    unsigned char* ib = ia + 32768;
+    unsigned char* ix = ib + 65536;
+    pack_tile_img_f16_kernel<<<(128 * 128 + 255) / 256, 256, 0, st>>>(A, (__half*)ia, 128, 128);
+    pack_tile_img_f16_kernel<<<(128 * 256 + 255) / 256, 256, 0, st>>>(B, (__half*)ib, 128, 256);
+    pack_tile_img_f16_kernel<<<(128 * 64 + 255) / 256, 256, 0, st>>>(X, (__half*)ix, 128, 64);
+    TOUED_LAUNCH_CHECK();
+    const size_t smem = 32768 + 65536 + 16384 + 1024;
+    TOUED_CUDA(cudaFuncSetAttribute(tc_gemm_mn_x16_test_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    tc_gemm_mn_x16_test_kernel<<<1, 128, smem, st>>>(ia, ib, ix, D);
+    TOUED_LAUNCH_CHECK();
+    return 0;
+}

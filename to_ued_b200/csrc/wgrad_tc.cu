@@ -1,12 +1,20 @@
-// Tensor-core weight gradient of the recurrent matrix:  dWh[j][c] = sum_tok h'[tok][j] * dGh[tok][c]
-// (the parameter-gradient sum of jax.grad through models/lpg.py:29, flax GRUCell hr/hz/hn kernels).
+// Tensor-core weight gradients of the GRU:  dWh[j][c] = sum_tok h'[tok][j] * dGh[tok][c]  and the input side
+// dWi[q][c], dbi[c], dbhn[c] = sum_tok x[tok][q] * dG[tok][c]  (the parameter-gradient sums of jax.grad through
+// models/lpg.py:29, flax GRUCell kernels and biases).
 //
-// Both operands are contracted over tokens, i.e. they are MN-major for tcgen05: the 64-token x 64-column
-// sub-tiles of the fp16 token tile images written by the forward (h') and backward (S * dG, tc.cuh) kernels are
-// bulk-copied (cp.async.bulk) into shared memory and used as-is.  A CTA owns one 128 (j) x 384 (c)
-// output tile (fp32 accumulators in 384 TMEM columns) and a contiguous range of token blocks; the four
-// tile types of one token range are adjacent CTAs so they share their operand stream through L2.
-// Output: per-split partial sums (deterministic; reduced by toued_reduce_partials).
+// Both operands are contracted over tokens, i.e. they are MN-major for tcgen05: the 64-token x 64-column sub-tiles of
+// the fp16 token tile images written by the forward (h', x) and backward (S * dG, tc.cuh) kernels are bulk-copied
+// (cp.async.bulk) into shared memory and used as-is.  The gate columns are the M side: a CTA computes
+// dWh^T = dG^T h' for one 128-column dG block (A: two dG sub-tiles) against all 256 hidden units (B: the four h'
+// sub-tiles, one M128 N256 K16 MMA per K-step), and with the same A descriptor  dG^T x  against the x sub-tile
+// (N = 16: the 8 real x rows and 8 zero columns of the image) into 16 more TMEM columns.  So the r, z and h_n blocks
+// (dG groups 0-11) yield dWh, dWi_r, dWi_z, dbi_r, dbi_z and dbhn from one dG stream.  The a_n block (groups 12-15)
+// only feeds dWi_n and dbi_n: the CTAs of column blocks 0-3 each also take one a_n group (x^T dG_an, M64 N64, of
+// which the 8 x rows are read).
+// A CTA owns one column block and one contiguous range of token blocks (a split); the six CTAs of one range are
+// adjacent so they share h' and x through L2.  Every output element is summed by one CTA over its split in token
+// order, K = 16 tokens per MMA, so the per-split partials (reduced by toued_reduce_partials) are deterministic, and on
+// B200 bitwise equal to those of the earlier kernel that had h' and x as A (same splits; DESIGN.md §7.0).
 #include "tc.cuh"
 #include "lpg_common.cuh"
 #include "../../include/toued.h"
@@ -16,7 +24,8 @@ constexpr int SMT_WI = 0, SMT_BHN = 8 * LPG_G, SMT_WPI = SMT_BHN + LPG_H, SMT_WY
               SMT_BPI = SMT_WY + LPG_H * LPG_Y, SMT_BY = SMT_BPI + 1, SMT_TOTAL = SMT_BY + LPG_Y;
 constexpr int WT_THREADS = 192;            // 4 epilogue warps + producer warp + MMA warp
 constexpr int WT_NS = 3;
-constexpr int WT_STAGE = 9 * 8192;         // dWh tiles: 2 A + 6 B sub-tiles of 8 KB; x tiles: 1 A + 8 B
+constexpr int WT_STAGE = 8 * 8192;         // 2 dG + 4 h' + 1 x (+ 1 a_n in column blocks 0-3) sub-tiles of 8 KB
+constexpr int WT_SPLITS = 24;              // 6 column blocks x 24 token splits = 144 CTAs
 
 __global__ void __launch_bounds__(WT_THREADS, 1)
 wgrad_wh_tc_kernel(const unsigned char* __restrict__ hpimg, const unsigned char* __restrict__ dgimg,
@@ -29,14 +38,13 @@ wgrad_wh_tc_kernel(const unsigned char* __restrict__ hpimg, const unsigned char*
     __shared__ __align__(8) uint64_t full[WT_NS], empty[WT_NS], done_bar;
     __shared__ uint32_t tmem_base_s;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    // tile types 0-3: dWh tile (jt, ct) = h'^T [128 j] x dG [384 c];
-    // tile types 4-5: input-side gradients  x^T [8 (of 64) inputs] x dG column groups 8*(type-4) .. +8
-    const int type = blockIdx.x % 6, split = blockIdx.x / 6;
-    const bool xt = type >= 4;
-    const int jt = (type >> 1) & 1, ct = type & 1;
+    // column block cb = dG groups 2cb, 2cb+1 (r: 0-1, z: 2-3, h_n: 4-5); cb < 4 also a_n group 12 + cb
+    const int cb = blockIdx.x % 6, split = blockIdx.x / 6;
+    const bool an = cb < 4;
     const int tb0 = split * blocks_per_split;
-    const int tb1 = min(n_tok_blocks, tb0 + blocks_per_split);
-    const int nblk = max(0, tb1 - tb0);
+    const int nblk = max(0, min(n_tok_blocks, tb0 + blocks_per_split) - tb0);
+    constexpr uint32_t H_OFF = 2 * 8192, X_OFF = 6 * 8192, AN_OFF = 7 * 8192;   // sub-tiles inside a stage
+    constexpr uint32_t T_X = 256, T_AN = 288;                                     // TMEM columns of the input side
 
     if (tid == 0) {
         for (int s = 0; s < WT_NS; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], 1); }
@@ -54,45 +62,34 @@ wgrad_wh_tc_kernel(const unsigned char* __restrict__ hpimg, const unsigned char*
             for (int i = 0; i < nblk; ++i) {
                 const int s = i % WT_NS;
                 mbar_wait(&empty[s], ((i / WT_NS) & 1) ^ 1);
-                mbar_expect_tx(&full[s], xt ? 9 * 8192 : 8 * 8192);
+                mbar_expect_tx(&full[s], an ? 8 * 8192 : 7 * 8192);
                 unsigned char* st = smem + s * WT_STAGE;
                 const size_t tb = (size_t)(tb0 + i);
-                if (!xt) {
-                    bulk_g2s(st, hpimg + ((tb * 4 + 2 * jt) << 13), 2 * 8192, &full[s]);            // j groups 2jt, 2jt+1
-                    bulk_g2s(st + 2 * 8192, dgimg + ((tb * 16 + 6 * ct) << 13), 6 * 8192, &full[s]);  // c groups 6ct .. 6ct+5
-                } else {
-                    bulk_g2s(st, ximg + (tb << 13), 8192, &full[s]);                                  // the x group
-                    bulk_g2s(st + 8192, dgimg + ((tb * 16 + 8 * ct) << 13), 7 * 8192, &full[s]);      // c groups 8ct .. 8ct+6
-                    bulk_g2s(st + 8 * 8192, dgimg + ((tb * 16 + 8 * ct + 7) << 13), 8192, &full[s]);  // c group 8ct+7
-                }
+                bulk_g2s(st, dgimg + ((tb * 16 + 2 * cb) << 13), 2 * 8192, &full[s]);      // dG groups 2cb, 2cb+1
+                bulk_g2s(st + H_OFF, hpimg + ((tb * 4) << 13), 4 * 8192, &full[s]);       // all 256 units of h'
+                bulk_g2s(st + X_OFF, ximg + (tb << 13), 8192, &full[s]);                  // the x group
+                if (an) bulk_g2s(st + AN_OFF, dgimg + ((tb * 16 + 12 + cb) << 13), 8192, &full[s]);   // a_n group
             }
         }
     } else if (warp == 5) {
         {   // all lanes wait, one elected lane issues (tc.cuh::elect_one)
-            constexpr uint32_t idesc = tc_idesc_mn(128, 192, 0), idesc_x = tc_idesc_mn(64, 256, 0);   // fp16; x tiles: M = 64 (one group, 8 rows used)
+            // fp16; TMEM lane = gate column.  x: N = 16 reads columns 0..15 of the 64-column x group (8 real + 8 zero);
+            // a_n: A = the x group with M = 64 (rows 0..7 used), TMEM lane = x row
+            constexpr uint32_t idesc = tc_idesc_mn(128, 256, 0), idesc_x = tc_idesc_mn(128, 16, 0),
+                               idesc_an = tc_idesc_mn(64, 64, 0);
             for (int i = 0; i < nblk; ++i) {
                 const int s = i % WT_NS;
                 mbar_wait(&full[s], (i / WT_NS) & 1);
                 tc_fence_after();
                 const uint32_t a0 = smem_u32(smem + s * WT_STAGE);
                 if (elect_one()) {
-                if (!xt) {
-                    const uint32_t b0 = a0 + 2 * 8192;
 #pragma unroll
-                    for (int ks = 0; ks < 4; ++ks) {
-                        const uint64_t ad = tc_smem_desc_mn(a0 + ks * 2048, 8192);
-                        tc_mma(tmem_base, ad, tc_smem_desc_mn(b0 + ks * 2048, 8192), idesc, (i | ks) != 0);
-                        tc_mma(tmem_base + 192, ad, tc_smem_desc_mn(b0 + 3 * 8192 + ks * 2048, 8192), idesc, (i | ks) != 0);
-                    }
-                } else {
-                    const uint32_t b0 = a0 + 8192;
-#pragma unroll
-                    for (int ks = 0; ks < 4; ++ks) {
-                        // M = 64: the single x group (halves the A fetch of these operand-fetch-bound MMAs)
-                        const uint64_t ad = tc_smem_desc_mn(a0 + ks * 2048, 0);
-                        tc_mma(tmem_base, ad, tc_smem_desc_mn(b0 + ks * 2048, 8192), idesc_x, (i | ks) != 0);
-                        tc_mma(tmem_base + 256, ad, tc_smem_desc_mn(b0 + 4 * 8192 + ks * 2048, 8192), idesc_x, (i | ks) != 0);
-                    }
+                for (int ks = 0; ks < 4; ++ks) {
+                    const uint32_t acc = (i | ks) != 0;
+                    const uint64_t ad = tc_smem_desc_mn(a0 + ks * 2048, 8192), xd = tc_smem_desc_mn(a0 + X_OFF + ks * 2048, 8192);
+                    tc_mma(tmem_base, ad, tc_smem_desc_mn(a0 + H_OFF + ks * 2048, 8192), idesc, acc);
+                    tc_mma(tmem_base + T_X, ad, xd, idesc_x, acc);
+                    if (an) tc_mma(tmem_base + T_AN, xd, tc_smem_desc_mn(a0 + AN_OFF + ks * 2048, 8192), idesc_an, acc);
                 }
                 tc_commit(&empty[s]);
                 }
@@ -102,73 +99,66 @@ wgrad_wh_tc_kernel(const unsigned char* __restrict__ hpimg, const unsigned char*
             __syncwarp();
         }
     } else {
-        // epilogue: TMEM lane = j within the tile
+        // epilogue: TMEM lane = gate column within the 128-column block
         mbar_wait(&done_bar, 0);
         tc_fence_after();
         // the dG image is in units of the launch's cotangent scale S (tc.cuh): take it back out of the fp32 sums
         const float inv_s = cotmax ? 1.0f / cot_scale_from_max(*cotmax) : 1.0f;
-        if (xt) {
-            // rows 0..7 of the x tile: dWi (rows q < X), dbi (row 7) and dbhn (row 7 of the dhn columns).
-            // Always accumulates: the head-gradient kernel has initialised this split's small-partial area.
-            if (warp == 0) {
-                float* out = small_partial + (size_t)split * SMT_TOTAL;
-                auto dst_of = [&](int cc) {
-                    if (ct == 0) return SMT_WI + lane * LPG_G + cc;                            // dar, daz columns
-                    if (cc >= 256) return SMT_WI + lane * LPG_G + 512 + (cc - 256);           // dan columns
-                    return lane == 7 ? SMT_BHN + cc : -1;                                     // sum of dhn
-                };
-                for (int c = 0; c < 512; c += 32) {          // 32 columns per round: loads first, then the stores
-                    float v[4][8], o[4][8];
+        const uint32_t trow = tmem_base + ((uint32_t)(warp * 32) << 16);
+        auto ld8 = [&](uint32_t col, float (&v)[8]) {             // 8 TMEM columns of this thread's lane (0 if no MMA ran)
+            if (nblk > 0) tmem_ld8(trow + col, v);
+            else {
 #pragma unroll
-                    for (int i = 0; i < 4; ++i) {
-                        if (nblk > 0) tmem_ld8(tmem_base + c + 8 * i, v[i]);
-                        else {
-#pragma unroll
-                            for (int e = 0; e < 8; ++e) v[i][e] = 0.f;
-                        }
-                    }
-                    if (nblk > 0) tmem_ld_wait();
-                    if (lane < 8) {
-#pragma unroll
-                        for (int i = 0; i < 4; ++i)
-#pragma unroll
-                            for (int e = 0; e < 8; ++e) { const int d = dst_of(c + 8 * i + e); o[i][e] = d >= 0 ? out[d] : 0.0f; }
-#pragma unroll
-                        for (int i = 0; i < 4; ++i)
-#pragma unroll
-                            for (int e = 0; e < 8; ++e) { const int d = dst_of(c + 8 * i + e); if (d >= 0) out[d] = fmaf(v[i][e], inv_s, o[i][e]); }
-                    }
-                }
+                for (int e = 0; e < 8; ++e) v[e] = 0.f;
             }
-        } else {
-        const int j = jt * 128 + warp * 32 + lane;
-        float* out = partial + (size_t)split * LPG_H * LPG_G + (size_t)j * LPG_G + ct * 384;
-        // 64 columns per round: the previous partials are fetched with 16 independent loads in flight
-        // (one dependent load -> add -> store round trip per 8 columns would serialise 48 DRAM latencies)
-        for (int c = 0; c < 384; c += 64) {
-            float4 pre[16];
-            float4* p = reinterpret_cast<float4*>(out + c);
-            if (accumulate) {
+        };
+        // input side, x row q (q < X: dWi, q = 7: the constant 1, i.e. the bias).  Always accumulates: the
+        // head-gradient kernel has initialised this split's small-partial area.
+        float* sp = small_partial + (size_t)split * SMT_TOTAL;
+        const int c = cb * 128 + warp * 32 + lane;
+        {
+            float v[8];
+            ld8(T_X, v);
+            if (nblk > 0) tmem_ld_wait();
+            if (cb < 4) {                                                        // r, z columns: dWi, dbi
+                float o[8];
 #pragma unroll
-                for (int i = 0; i < 16; ++i) pre[i] = p[i];
-            } else {
+                for (int q = 0; q < 8; ++q) o[q] = sp[SMT_WI + q * LPG_G + c];
 #pragma unroll
-                for (int i = 0; i < 16; ++i) pre[i] = make_float4(0.f, 0.f, 0.f, 0.f);
-            }
-#pragma unroll
-            for (int i = 0; i < 8; ++i) {
-                float v[8];
-                if (nblk > 0) {
-                    tmem_ld8(tmem_base + ((uint32_t)(warp * 32) << 16) + c + 8 * i, v);
-                    tmem_ld_wait();
-                } else {
-#pragma unroll
-                    for (int e = 0; e < 8; ++e) v[e] = 0.f;
-                }
-                p[2 * i] = make_float4(fmaf(v[0], inv_s, pre[2 * i].x), fmaf(v[1], inv_s, pre[2 * i].y), fmaf(v[2], inv_s, pre[2 * i].z), fmaf(v[3], inv_s, pre[2 * i].w));
-                p[2 * i + 1] = make_float4(fmaf(v[4], inv_s, pre[2 * i + 1].x), fmaf(v[5], inv_s, pre[2 * i + 1].y), fmaf(v[6], inv_s, pre[2 * i + 1].z), fmaf(v[7], inv_s, pre[2 * i + 1].w));
+                for (int q = 0; q < 8; ++q) sp[SMT_WI + q * LPG_G + c] = fmaf(v[q], inv_s, o[q]);
+            } else {                                                             // h_n columns: only dbhn (x row 7)
+                sp[SMT_BHN + c - 2 * LPG_H] = fmaf(v[7], inv_s, sp[SMT_BHN + c - 2 * LPG_H]);
             }
         }
+        if (an) {                       // a_n group 12 + cb: TMEM lane q < 8 (warp 0) = x row, column = a_n column
+            float v[8][8];
+#pragma unroll
+            for (int i = 0; i < 8; ++i) ld8(T_AN + 8 * i, v[i]);                // (collective: the whole warp loads)
+            if (nblk > 0) tmem_ld_wait();
+            if (warp == 0 && lane < 8) {
+                float* dst = sp + SMT_WI + lane * LPG_G + 2 * LPG_H + 64 * cb;
+                float o[8][8];
+#pragma unroll
+                for (int i = 0; i < 8; ++i)
+#pragma unroll
+                    for (int e = 0; e < 8; ++e) o[i][e] = dst[8 * i + e];
+#pragma unroll
+                for (int i = 0; i < 8; ++i)
+#pragma unroll
+                    for (int e = 0; e < 8; ++e) dst[8 * i + e] = fmaf(v[i][e], inv_s, o[i][e]);
+            }
+        }
+        // dWh: partial[split][j][c]; a warp's lanes are 32 consecutive c, so every access is one 128-byte line
+        float* out = partial + (size_t)split * LPG_H * LPG_G + c;
+        for (int j0 = 0; j0 < LPG_H; j0 += 32) {          // 32 previous partials in flight, then the stores
+            float pre[32], w[4][8];
+#pragma unroll
+            for (int e = 0; e < 32; ++e) pre[e] = accumulate ? out[(size_t)(j0 + e) * LPG_G] : 0.0f;
+#pragma unroll
+            for (int i = 0; i < 4; ++i) ld8(j0 + 8 * i, w[i]);
+            if (nblk > 0) tmem_ld_wait();
+#pragma unroll
+            for (int e = 0; e < 32; ++e) out[(size_t)(j0 + e) * LPG_G] = fmaf(w[e >> 3][e & 7], inv_s, pre[e]);
         }
     }
     tc_fence_before();
@@ -282,7 +272,7 @@ wgrad_heads_stream_kernel(const __half* __restrict__ h16, const float* __restric
             if (lane == 16 + i) put(SMT_BPI + i, v);
         }
     }
-    if (!accumulate) {                    // the x-tile CTAs of the GEMM kernel add into the input-side area
+    if (!accumulate) {                    // the input-side MMAs of the GEMM kernel add into this area
         for (int i = blockIdx.x * 256 + threadIdx.x; i < SMT_WPI; i += 4 * 256) out[i] = 0.0f;
     }
 }
@@ -457,7 +447,7 @@ wgrad_heads_mma_kernel(const __half* __restrict__ h16, const float* __restrict__
                 if (lane == i) out[SMT_BPI + i] = accumulate ? out[SMT_BPI + i] + v : v;
             }
         }
-        if (!accumulate) {                // the x-tile CTAs of the GEMM kernel add into the input-side area
+        if (!accumulate) {                // the input-side MMAs of the GEMM kernel add into this area
             for (int i = tid; i < SMT_WPI; i += 128) out[i] = 0.0f;
         }
     }
@@ -466,8 +456,8 @@ wgrad_heads_mma_kernel(const __half* __restrict__ h16, const float* __restrict__
     if (warp == 5) tmem_dealloc(tmem_base, 64);
 }
 
-constexpr int WT_SPLITS = 24;              // 6 tile types x 24 = 144 CTAs
 static_assert(WT_SPLITS <= 37 && HT_SPLITS <= 592, "partial areas of toued_lpg_wgrad_workspace_floats (lpg_backward.cu) are sized for 37 / 592 splits");
+static_assert(WT_SPLITS <= HT_SPLITS, "the GEMM adds into small-partial areas the head-gradient kernel initialises");
 extern "C" int toued_wgrad_tc_splits(void) { return WT_SPLITS; }
 extern "C" int toued_wgrad_tc_small_splits(void) { return HT_SPLITS; }
 
@@ -481,7 +471,7 @@ extern "C" int toued_lpg_wgrad_tc(const void* hpimg, const void* dgimg, const vo
     const int Rp = (R + 63) / 64 * 64;
     const int n_tb = L * Rp / 64;
     const int bps = (n_tb + WT_SPLITS - 1) / WT_SPLITS;
-    // head gradients first: also zero-initialises the input-side area the GEMM's x tiles accumulate into
+    // head gradients first: also zero-initialises the input-side area the GEMM's x MMAs accumulate into
     const int nrb = L * ((R + 31) / 32);
     const int rbps = (nrb + HT_SPLITS - 1) / HT_SPLITS;
     if (R % 32 == 0) {
